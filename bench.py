@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — VSS env-steps/s (and PPO SPS) on N B200s, with roofline, CPU baseline and e2e.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--envs E_PER_GPU] [--impl native|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--envs E_PER_GPU] [--impl native|reference] [--dump-outputs DIR]
   torchrun --nproc-per-node N bench.py --gpus N ...        (one rank per GPU, NCCL only for timing / PPO grads)
 
 A "step" is one pass of the hot path over one batch: one fused `vss_step` launch advancing E
@@ -37,6 +37,8 @@ sys.path.insert(0, ROOT)
 BYTES_PER_FIELD_STEP = 240 + 240 + 48 + 8 + 8 + 1248 + 1248 + 96 + 1 + 4
 # host bytes of the full contract per field-step: actions in; obs, terminal obs, rewards, reset, timeout, progress out
 FULL_H2D, FULL_D2H = 48, 1248 + 1248 + 96 + 8 + 1 + 4
+# fields sampled by --dump-outputs: 2.6 KB of outputs per field keeps a dump near 43 MB
+DUMP_FIELDS = 16384
 
 
 def parse():
@@ -58,7 +60,14 @@ def parse():
                     help="updates per PPO leg (1 eager + 1 capturing + steady); 0 = about 2e7 samples per GPU and leg, "
                          "at least 8 and at most 40 updates, so that the reference's own SPS metric (global_step / wall, "
                          "start-up included) is not dominated by the two start-up updates")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed VSS.step returned as DIR/<name>.npy "
+                         f"(float32 / float64; the same {DUMP_FIELDS} sampled fields in every run, all fields when "
+                         "there are fewer; rank 0's fields)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs dumps the native arm's outputs: use it with --impl native")
+    return args
 
 
 # ----------------------------------------------------------------------------- clocks
@@ -265,6 +274,25 @@ def full_contract_host_step(torch, envs, local):
     return step
 
 
+def dump_outputs(torch, out_dir, step_out):
+    """Writes what one `VSS.step` returned, `(obs_dict, rew, reset, extras)`, as out_dir/<name>.npy: floats as
+    float32, the int64 reset flags as float64 (exact), the bool time-outs as float32 0 / 1. Fields beyond
+    DUMP_FIELDS are sampled with a fixed seed, so two runs with the same arguments dump the same fields."""
+    import numpy as np
+    obs, rew, reset, extras = step_out
+    arrays = {"obs": obs["obs"], "rew": rew, "reset": reset, "terminal_observation": extras["terminal_observation"],
+              "time_outs": extras["time_outs"], "progress_buffer": extras["progress_buffer"]}
+    n = reset.shape[0]
+    rows = None
+    if n > DUMP_FIELDS:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_FIELDS, replace=False))
+        rows = torch.from_numpy(rows).to(reset.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = (t if rows is None else t.index_select(0, rows)).cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64 if a.dtype == np.int64 else np.float32))
+
+
 def reference_torch_legs(torch, peak):
     """BASELINE.md B2-B4: the reference's own torch code paths (restated, oracle/torch_ref.py) on this GPU."""
     import types
@@ -385,14 +413,22 @@ def run_native(args):
     envs, acts = make_task(torch, n, rank, local)
 
     def step_full(i):
-        envs.step(acts[i & 3])  # the drop-in VSS.step: one fused vss_step launch
+        return envs.step(acts[i & 3])  # the drop-in VSS.step: one fused vss_step launch
+
+    last = {}
+
+    def timed_step(i):
+        last["out"] = step_full(i)
 
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()   # before the warm-up; `mark` drops the warm-up samples when the timed region starts
-    ms = time_steps(torch, dist, world, step_full, args.steps, args.warmup, on_start=sampler.mark)
+    ms = time_steps(torch, dist, world, timed_step, args.steps, args.warmup, on_start=sampler.mark)
     clocks = sampler.stop() if rank == 0 else None
     value = world * n * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:   # before the legs below step the same fields again
+        dump_outputs(torch, args.dump_outputs, last["out"])
+    last.clear()
 
     peaks = {}
     try:

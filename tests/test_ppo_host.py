@@ -1,6 +1,7 @@
 """CPU: host-side PPO logic against golden vectors from the reference's own script."""
 import json
 import os
+import sys
 import types
 
 import numpy as np
@@ -9,6 +10,9 @@ import torch
 
 from conftest import GOLDEN
 from rsoccer_isaac_cleanrl_b200 import ppo
+
+sys.path.insert(0, GOLDEN)
+import make_golden as mg  # noqa: E402  (checksum helpers only; the reference is not read here)
 
 
 def test_cli_flags_and_defaults_match_reference():
@@ -30,8 +34,22 @@ def _envs(adim):
 
 def test_agent_state_dict_loads_reference_checkpoint_and_matches_outputs():
     z = np.load(os.path.join(GOLDEN, "agent.npz"))
-    agent = ppo.Agent(_envs(2))
+    # the hidden 256/512-wide weights are not stored: rebuilt from the generator's seed with this Agent (same layer
+    # order and initialisers), then pinned to the reference's by per-tensor checksum and a strided sample; one
+    # thread, as the generator ran: orthogonal_'s QR rounds differently with more
+    threads = torch.get_num_threads()
+    torch.set_num_threads(1)
+    try:
+        torch.manual_seed(3)
+        rebuilt = ppo.Agent(_envs(2)).state_dict()
+    finally:
+        torch.set_num_threads(threads)
     sd = {k[len("a2_sd_"):]: torch.from_numpy(z[k]) for k in z.files if k.startswith("a2_sd_")}
+    for k in (k[len("a2_sum_"):] for k in z.files if k.startswith("a2_sum_")):
+        np.testing.assert_allclose(mg.weight_checksum(rebuilt[k]), z[f"a2_sum_{k}"], rtol=1e-9, err_msg=k)
+        np.testing.assert_array_equal(mg.weight_sample(rebuilt[k]), z[f"a2_sample_{k}"], err_msg=k)
+        sd[k] = rebuilt[k]
+    agent = ppo.Agent(_envs(2))
     assert set(sd) == set(agent.state_dict())           # same keys as the reference's Agent
     agent.load_state_dict(sd, strict=True)
     x, action = torch.from_numpy(z["a2_x"]), torch.from_numpy(z["a2_action"])
