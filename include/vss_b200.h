@@ -266,6 +266,53 @@ VSS_API int vss_set_step_fields_per_tile(vss_handle h, int fields);
 VSS_API int vss_step_fields_per_tile(vss_handle h);
 VSS_API int vss_set_step_range(vss_handle h, int64_t first_field, int64_t num_fields);
 
+/* ---- match evaluation: play.py::play_matches (reference play.py:131-164) on the device ----
+ * One team per side, each driving its 6 action slots of the (N,2,3,2) buffer in one of these modes
+ * (reference play.py:26-64):
+ *   ZERO      TeamZero: act[:] *= 0 (the previous values times 0: the sign of zero is kept)
+ *   OU        TeamOU: the OU draw (wrappers.py:5-19)
+ *   SA        TeamSA: the OU draw, then robot 0 = policy_action (N,2)
+ *   CMA       TeamCMA: the 6 slots = policy_action (N,6)
+ *   DMA       TeamDMA / ppo-sa-x3: the 6 slots = policy_action (3N,2) (= (N,6))
+ *   EXTERNAL  any other team: the slots are left as the caller wrote them into the buffer */
+#define VSS_TEAM_ZERO 0
+#define VSS_TEAM_OU 1
+#define VSS_TEAM_SA 2
+#define VSS_TEAM_CMA 3
+#define VSS_TEAM_DMA 4
+#define VSS_TEAM_EXTERNAL 5
+typedef struct vss_match_team {
+  int32_t mode;                /* VSS_TEAM_* */
+  int32_t reserved;
+  const float* policy_action;  /* SA (N,2), CMA (N,6), DMA (3N,2) f32; required by those modes, ignored otherwise */
+  void* rows_bf16;             /* SA / CMA (N,64), DMA (3N,64) bf16, or NULL: the team's rows of the post-reset
+                                  observation (robot 0, or robots 0-2; yellow = the mirrored obs[:,1] rows) rounded
+                                  to nearest even, columns 52..63 never written - the input of the team's next
+                                  policy call. Ignored by the other modes. */
+} vss_match_team;
+/* Scoreboard of a match evaluation (device memory, 40 bytes, zeroed by the caller before the first step):
+ * the statistics the reference's loop accumulates (play.py:152-164). */
+typedef struct vss_match_board {
+  int64_t matches;     /* episodes that ended among the fields < count_envs, counted while not frozen */
+  int64_t length_sum;  /* sum of their un-reset progress counters (info["progress_buffer"]) */
+  double score_sum;    /* sum of their rew[env,0,0,0]: the goal term of blue robot 0 with the weights as set */
+  int64_t steps;       /* steps counted, the one that froze the board included */
+  uint32_t frozen;     /* set at the end of the step in which `matches` reached n_matches; later steps count
+                          nothing, so a caller may run steps past it (a captured chunk) without changing the
+                          result: score = score_sum / matches, length = length_sum / matches */
+  uint32_t reserved;
+} vss_match_board;
+/* One step of a two-team match: what play_matches does per iteration (both team calls + VSS.step +
+ * the statistics), in one launch. The action prologue reads action_buf, draws the views' OU noise
+ * (Philox stream 2 keyed by the device step index) on all 12 slots, applies each team's mode, stores
+ * the buffer back un-clamped and clamps it into the state; a done field's row is NOT zeroed (play_matches
+ * carries the OU state across resets). Outputs: reset_buf (io, as vss_step), the teams' bf16 rows, obs
+ * (N,2,3,52) f32 post-reset (may be NULL: only EXTERNAL teams need it) and the scoreboard. No terminal
+ * observation, no f32 rewards. Advances the step index like vss_step_view. Whole-engine launches only:
+ * rejected while vss_set_step_range is active. */
+VSS_API int vss_step_match(vss_handle h, const vss_match_team teams[2], float* action_buf, int64_t* reset_buf,
+                           float* obs, int64_t count_envs, int64_t n_matches, vss_match_board* board, void* stream);
+
 /* State access for parity tests and checkpointing: copies the SoA state
  * (VSS_STATE_WORDS x ld 32-bit words) device->device. */
 VSS_API int vss_get_state(vss_handle h, float* state_out, void* stream);

@@ -60,6 +60,19 @@ class ConvertJob(C.Structure):
 
 MAX_CONVERT_JOBS = 8
 
+TEAM_ZERO, TEAM_OU, TEAM_SA, TEAM_CMA, TEAM_DMA, TEAM_EXTERNAL = 0, 1, 2, 3, 4, 5
+
+
+class MatchTeam(C.Structure):
+    """`vss_match_team` of include/vss_b200.h."""
+
+    _fields_ = [("mode", C.c_int32), ("reserved", C.c_int32), ("policy_action", C.c_void_p), ("rows_bf16", C.c_void_p)]
+
+
+# `vss_match_board` of include/vss_b200.h as int64 words: matches, length_sum, score_sum (float64 bits), steps,
+# frozen (low 32 bits)
+BOARD_WORDS = 5
+
 
 class MlpSampling(C.Structure):
     """`vss_mlp_sampling` of include/vss_b200.h."""
@@ -97,6 +110,7 @@ _SYMBOLS = {
     "vss_set_step_fields_per_tile": (C.c_int, [_VP, C.c_int]),
     "vss_step_fields_per_tile": (C.c_int, [_VP]),
     "vss_set_step_range": (C.c_int, [_VP, C.c_int64, C.c_int64]),
+    "vss_step_match": (C.c_int, [_VP, C.POINTER(MatchTeam), _VP, _VP, _VP, C.c_int64, C.c_int64, _VP, _VP]),
     "vss_get_state": (C.c_int, [_VP, _VP, _VP]),
     "vss_set_state": (C.c_int, [_VP, _VP, _VP]),
     "vss_step_count": (C.c_uint64, [_VP]),

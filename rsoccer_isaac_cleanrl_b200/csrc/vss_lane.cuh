@@ -827,6 +827,7 @@ VSS_HD void st_bf16x4(void* base, long long off, const F4& v) {
 #endif
 
 constexpr int VIEW_FULL = -1;
+constexpr int VIEW_MATCH = 3;  // vss_step_match: two teams, the scoreboard, no terminal observation / f32 rewards
 
 struct StepArgs {
   float* state; long long n, ld; unsigned long long goff;  // n = end of the field range of this launch
@@ -856,11 +857,19 @@ struct StepArgs {
   void* packed;
   int fpw;                     // fields per warp: 32, or 16 / 8 for small batches (idle lanes, shorter critical path)
   int stagger_ns;              // first-wave CTAs start (blockIdx / 148 % 6) * stagger_ns late (0 = off)
+  // match mode only (vss_step_match): per team (blue, yellow) its VSS_TEAM_* mode, policy action and bf16 rows; the
+  // scoreboard counts the episodes of the fields < count_envs until n_matches
+  int team_mode[2];
+  const float* team_action[2];
+  void* team_rows[2];
+  long long count_envs, n_matches;
+  vss_match_board* board;
 };
 
 template <int VIEW>
 struct ViewShape {
-  static constexpr int F4_PER = VIEW == VIEW_FULL ? F4_PER_FIELD : (VIEW == VSS_VIEW_DMA ? 3 * F4_PER_ROW : F4_PER_ROW);
+  static constexpr int F4_PER = (VIEW == VIEW_FULL || VIEW == VIEW_MATCH) ? F4_PER_FIELD
+                                                                          : (VIEW == VSS_VIEW_DMA ? 3 * F4_PER_ROW : F4_PER_ROW);
   static constexpr int AGENTS = VIEW == VSS_VIEW_DMA ? 3 : 1;  // view "envs" per field
 };
 
@@ -888,6 +897,25 @@ VSS_HD void store_state(const float* S, float* state, long long ld, long long en
   for (int w = 0; w < VSS_STATE_WORDS; ++w) dst[(long long)w * ld] = S[w * LDS];
 }
 
+// Match mode: does either team draw OU noise (TeamOU, and robots 1-2 of TeamSA)?
+VSS_HD bool match_needs_ou(const StepArgs& a) {
+  return a.team_mode[0] == VSS_TEAM_OU || a.team_mode[0] == VSS_TEAM_SA || a.team_mode[1] == VSS_TEAM_OU ||
+         a.team_mode[1] == VSS_TEAM_SA;
+}
+// Match mode: action slot s (0..11) of the field after its team's call (play.py:34-64), given the buffer's previous
+// value and the OU draw of the slot.
+VSS_HD float match_slot(const StepArgs& a, long long env, int s, float prev, float ou) {
+  const int t = s >= 6 ? 1 : 0, k = s - 6 * t;
+  switch (a.team_mode[t]) {
+    case VSS_TEAM_ZERO: return fmul(prev, 0.0f);  // act[:] *= 0 keeps the sign of zero
+    case VSS_TEAM_OU: return ou;
+    case VSS_TEAM_SA: return k < 2 ? a.team_action[t][2 * env + k] : ou;
+    case VSS_TEAM_CMA:
+    case VSS_TEAM_DMA: return a.team_action[t][6 * env + k];  // (N,6) and (3N,2): the same 6 floats per field
+    default: return prev;                                      // EXTERNAL: as the caller wrote it
+  }
+}
+
 // Phase 1a of a step for one field: state in, actions (+OU noise), progress restart, prev clones.
 template <int VIEW>
 VSS_HD void lane_phase1a(float* S, long long env, const StepArgs& a, const DevParams& P, const RngKey& key) {
@@ -903,7 +931,18 @@ VSS_HD void lane_phase1a(float* S, long long env, const StepArgs& a, const DevPa
       act[4 * q] = v.x; act[4 * q + 1] = v.y; act[4 * q + 2] = v.z; act[4 * q + 3] = v.w;
     }
   }
-  if (VIEW != VIEW_FULL) {
+  if (VIEW == VIEW_MATCH) {
+    float ou[VSS_ACT_PER_FIELD];
+#pragma unroll
+    for (int q = 0; q < VSS_ACT_PER_FIELD; ++q) ou[q] = act[q];
+    if (match_needs_ou(a)) ou_lane(ou, P, key, step_index(a));
+#pragma unroll
+    for (int q = 0; q < VSS_ACT_PER_FIELD; ++q) act[q] = match_slot(a, env, q, act[q], ou[q]);
+    // the buffer keeps the un-clamped values; done rows are NOT zeroed (play_matches carries them over)
+    float* ap = a.action_buf + env * VSS_ACT_PER_FIELD;
+#pragma unroll
+    for (int q = 0; q < 3; ++q) st4(ap + 4 * q, F4{act[4 * q], act[4 * q + 1], act[4 * q + 2], act[4 * q + 3]});
+  } else if (VIEW != VIEW_FULL) {
     ou_lane(act, P, key, step_index(a));  // action_buf = random_ou(action_buf)
     if (VIEW == VSS_VIEW_SA) {     // act_view[:] = action
       act[0] = a.policy_action[2 * env]; act[1] = a.policy_action[2 * env + 1];
@@ -950,7 +989,13 @@ VSS_HD void actions_block(float* S, long long env, const StepArgs& a, const DevP
   float* ab = const_cast<float*>(VIEW == VIEW_FULL ? a.actions : a.action_buf) + env * VSS_ACT_PER_FIELD + 4 * b;
   const F4 v = ld4(ab);
   float act[4] = {v.x, v.y, v.z, v.w};
-  if (VIEW != VIEW_FULL) {
+  if (VIEW == VIEW_MATCH) {
+    float ou[4] = {v.x, v.y, v.z, v.w};
+    if (match_needs_ou(a)) ou_block(ou, P, key, step_index(a), (uint32_t)b);
+#pragma unroll
+    for (int q = 0; q < 4; ++q) act[q] = match_slot(a, env, 4 * b + q, act[q], ou[q]);
+    st4(ab, F4{act[0], act[1], act[2], act[3]});
+  } else if (VIEW != VIEW_FULL) {
     ou_block(act, P, key, step_index(a), (uint32_t)b);
     if (VIEW == VSS_VIEW_SA) {
       if (b == 0) { act[0] = a.policy_action[2 * env]; act[1] = a.policy_action[2 * env + 1]; }
@@ -1022,11 +1067,62 @@ VSS_HD_COLD void lane_sanitise(float* S, const StepArgs& a, const DevParams& P, 
   reset_lane(S, P, key);
   count_sanitised(a);
 }
+// ---- match scoreboard (vss_match_board): adds of the fields during a step, frozen by the end of the step ----
+VSS_HD bool board_frozen(const StepArgs& a) {
+#if defined(__CUDA_ARCH__)
+  return __ldcg(&a.board->frozen) != 0u;  // set by the last CTA of an earlier launch: read at L2
+#else
+  return a.board->frozen != 0u;
+#endif
+}
+VSS_HD void board_add(const StepArgs& a, float score, int progress) {
+#if defined(__CUDA_ARCH__)
+  atomicAdd(reinterpret_cast<unsigned long long*>(&a.board->matches), 1ull);
+  atomicAdd(reinterpret_cast<unsigned long long*>(&a.board->length_sum), (unsigned long long)progress);
+  atomicAdd(&a.board->score_sum, (double)score);
+#else
+#pragma omp atomic
+  a.board->matches += 1;
+#pragma omp atomic
+  a.board->length_sum += progress;
+#pragma omp atomic
+  a.board->score_sum += (double)score;
+#endif
+}
+// Called once per step after every field's adds: the step counts, and the board freezes once the count is reached
+// (play.py:152: the loop stops after the step in which ep_count reaches n_matches, with all of that step's dones).
+VSS_HD void board_close_step(volatile vss_match_board* b, long long n_matches) {
+  if (b->frozen) return;
+  b->steps = b->steps + 1;
+  if (b->matches >= n_matches) b->frozen = 1u;
+}
+
+// Match mode: dones and the scoreboard (play.py:152-160). A field < count_envs whose episode ended adds its
+// rew[env,0,0,0] (the goal term of blue robot 0, as rewards_lane computes it) and its un-reset progress.
+VSS_HD int match_outputs(const float* S, long long env, const StepArgs& a, const DevParams& P, bool finite,
+                         int progress) {
+  const bool goal = is_goal(S[0], S[LDS], P);
+  const bool done = !finite || goal || progress >= P.max_len;
+  a.reset_buf[env] = done ? 1 : 0;
+  if (done && env < a.count_envs && !board_frozen(a)) {
+    float score = 0.0f;
+    if (finite && P.w_goal > 0.0f) {
+      float gv = 0.0f;
+      if (goal && S[0] > 0.0f) gv = 1.0f;
+      if (goal && S[0] < 0.0f) gv = -1.0f;
+      score = fmul(gv, P.w_goal);
+    }
+    board_add(a, score, progress);
+  }
+  return !done ? LANE_RUNNING : (finite ? LANE_DONE : LANE_SANITISED);
+}
+
 template <int VIEW>
 VSS_HD int lane_outputs(float* S, long long env, const StepArgs& a, const DevParams& P, bool finite) {
   constexpr int AGENTS = ViewShape<VIEW>::AGENTS;
   const int progress = (int)fbits(S[VSS_W_PROGRESS * LDS]) + 1;
   S[VSS_W_PROGRESS * LDS] = bitsf((uint32_t)progress);
+  if (VIEW == VIEW_MATCH) return match_outputs(S, env, a, P, finite, progress);
   float rew[VSS_REW_PER_FIELD];
   if (finite) {
     rewards_lane(S, P, rew);
@@ -1098,7 +1194,7 @@ VSS_HD void zero_action_row(long long env, const StepArgs& a) {
 template <int VIEW>
 VSS_HD void lane_phase5(const float* S, long long env, const StepArgs& a, bool done) {
   store_state(S, a.state, a.ld, env);
-  if (VIEW != VIEW_FULL && done) zero_action_row(env, a);
+  if (VIEW != VIEW_FULL && VIEW != VIEW_MATCH && done) zero_action_row(env, a);
 }
 
 // Cooperative, coalesced observation write of one tile (all 32 lanes call it).
@@ -1209,6 +1305,27 @@ VSS_HD void write_obs_fields(const float* T, const uint32_t* tab, int lane, int 
       if (obh) st_bf16x4(obh, bf16_pad_offset(e * per_field + j), v);
       if (pk) st_bf16x4(pk, packed_offset(e * per_field + j), v);
     }
+  }
+}
+
+// Match mode: the post-reset observation of the tile's fields (cooperative, all 32 lanes of `parts` warps): the f32
+// (N,2,3,52) obs when a.obs is set, and each policy team's bf16 rows (SA / CMA: robot 0 -> row env; DMA: robot i ->
+// row 3 env + i; the yellow rows are the mirrored obs[:,1] rows). Slots that go nowhere are not gathered.
+VSS_HD void write_match_tile(const float* T, const uint32_t* tab, int lane, int valid, long long env0, const StepArgs& a,
+                             int part = 0, int parts = 1) {
+  const int total = valid * F4_PER_FIELD;
+  for (int f = lane + 32 * part; f < total; f += 32 * parts) {
+    const int e = f / F4_PER_FIELD, j = f - e * F4_PER_FIELD;
+    const int row = j / F4_PER_ROW, t = row / 3, i = row - 3 * t;
+    const int m = a.team_mode[t];
+    void* rows = a.team_rows[t];
+    long long r = -1;  // the team's bf16 row of this slot
+    if (rows && m == VSS_TEAM_DMA) r = 3 * (env0 + e) + i;
+    else if (rows && i == 0 && (m == VSS_TEAM_SA || m == VSS_TEAM_CMA)) r = env0 + e;
+    if (!a.obs && r < 0) continue;
+    const F4 v = obs_gather(T, tab[j], e);
+    if (a.obs) st4(a.obs + 4 * (env0 * F4_PER_FIELD + f), v);
+    if (r >= 0) st_bf16x4(rows, r * 64 + (j - row * F4_PER_ROW) * 4, v);
   }
 }
 

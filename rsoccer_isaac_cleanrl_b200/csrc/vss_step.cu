@@ -89,11 +89,20 @@ __device__ __forceinline__ unsigned long long globaltimer_ns() {
 // has read the step index (phase 1a) by then. The CTA that completes the step — `a.grid` CTAs, over all
 // the range launches of one step — clears the count and advances the step index (step_ctr[0]); launches
 // of the next step are ordered after every launch of this one, so they read the new index.
+// Match mode: every thread fences its scoreboard adds before its warp is counted, and the completing CTA fences
+// again before it reads the count and closes the step (the last-block pattern of a threadfence reduction).
+template <int VIEW>
 __device__ __forceinline__ void step_done(const StepArgs& a, uint32_t* ctr) {
+  if (VIEW == VIEW_MATCH) __threadfence();
   __syncwarp();
   if ((threadIdx.x & 31) == 0 && atomicAdd(&ctr[3], 1u) == (blockDim.x >> 5) - 1u) {
+    if (VIEW == VIEW_MATCH) __threadfence();
     unsigned long long* done_ctas = a.step_ctr + 1;
     if (atomicAdd(done_ctas, 1ull) == (unsigned long long)a.grid - 1ull) {
+      if (VIEW == VIEW_MATCH) {
+        __threadfence();
+        board_close_step(a.board, a.n_matches);
+      }
       atomicExch(done_ctas, 0ull);
       atomicAdd(a.step_ctr, 1ull);
     }
@@ -125,7 +134,7 @@ k_step(const __grid_constant__ StepArgs a, const __grid_constant__ DevParams P) 
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const long long tile = (long long)blockIdx.x * (blockDim.x >> 5) + warp;
   const long long env0 = a.env_begin + tile * a.fpw;
-  if (!SYNC && env0 >= a.n) { if (VIEW != VIEW_FULL) step_done(a, ctr); return; }  // (with block-level syncs every warp stays until the end)
+  if (!SYNC && env0 >= a.n) { if (VIEW != VIEW_FULL) step_done<VIEW>(a, ctr); return; }  // (with block-level syncs every warp stays until the end)
   float* T = tiles + warp * TILE_STATE_WORDS;
   float* S = T + lane;
   const long long env = env0 + lane;
@@ -154,20 +163,22 @@ k_step(const __grid_constant__ StepArgs a, const __grid_constant__ DevParams P) 
   void* pk = (VIEW != VIEW_FULL && a.packed)
                  ? static_cast<void*>(static_cast<char*>(a.packed) + env0 * (ViewShape<VIEW>::AGENTS * VSS_PACKED_ROW_BYTES))
                  : nullptr;
-  if (PER_FIELD >= 32) write_obs_tile_rows<PER_FIELD>(T, tab, lane, valid, tob, ob, done_mask, obh, pk);
+  if (VIEW == VIEW_MATCH) {}  // (no terminal observation: every row is written once, after the reset)
+  else if (PER_FIELD >= 32) write_obs_tile_rows<PER_FIELD>(T, tab, lane, valid, tob, ob, done_mask, obh, pk);
   else write_obs_tile(T, tab, lane, valid, PER_FIELD, tob, ob, done_mask, obh, pk);
   __syncwarp();
   // 3. masked reset (vss.py:202, 267-333)
   if (done) reset_lane(S, P, key);
   __syncwarp();
   // 4. observation of the fields that were reset (vss.py:203)
-  write_obs_fields(T, tab, lane, PER_FIELD, ob, done_mask, obh, pk);
+  if (VIEW == VIEW_MATCH) write_match_tile(T, tab, lane, valid, env0, a);
+  else write_obs_fields(T, tab, lane, PER_FIELD, ob, done_mask, obh, pk);
   // 5. state out
   if (SYNC) __syncthreads();
   if (active) lane_phase5<VIEW>(S, env, a, code != LANE_RUNNING);
   // only the views draw OU noise: the full-contract step neither reads nor advances the index (the
   // extra memory operation at the end of every CTA costs 1 % of the launch at 2^20 fields)
-  if (VIEW != VIEW_FULL) step_done(a, ctr);
+  if (VIEW != VIEW_FULL) step_done<VIEW>(a, ctr);
 }
 
 // ----------------------------------------------------------------------------------------
@@ -325,6 +336,8 @@ k_step_cta(const __grid_constant__ StepArgs a, const __grid_constant__ DevParams
     const uint32_t dm = __ballot_sync(0xffffffffu, code == LANE_DONE);      // needs the masked reset of phase 3
     const uint32_t em = __ballot_sync(0xffffffffu, code != LANE_RUNNING);  // episode ended (done or sanitised)
     if (lane == 0) { ctr[0] = dm; ctr[1] = em; }
+  } else if (VIEW == VIEW_MATCH) {
+    // (no terminal observation: every row is written once, after the reset)
   } else if (PER_FIELD >= 32) {
     write_obs_tile_rows<PER_FIELD, true>(T, tab, lane, valid, tob, ob, 0u, obh, pk, warp - 1, NW - 1);
   } else {
@@ -339,11 +352,14 @@ k_step_cta(const __grid_constant__ StepArgs a, const __grid_constant__ DevParams
       if (w != VSS_W_PROGRESS) S[w * LDS] = Sh[w * LDS];
   __syncthreads();
   // 4. observation of the fields that were reset (vss.py:203); 5. state out
-  write_obs_fields(T, tab, lane, PER_FIELD, ob, done_mask, obh, pk, warp, NW);
+  if (VIEW == VIEW_MATCH) write_match_tile(T, tab, lane, valid, env0, a, warp, NW);
+  else write_obs_fields(T, tab, lane, PER_FIELD, ob, done_mask, obh, pk, warp, NW);
   if (active) store_state_words(S, a.state, a.ld, env, warp, NW);
-  if (VIEW != VIEW_FULL) {
+  if (VIEW == VIEW_MATCH) {
+    step_done<VIEW>(a, ctr);  // (done rows keep their actions: play_matches carries the OU state over)
+  } else if (VIEW != VIEW_FULL) {
     if (warp == 0 && ((ended_mask >> lane) & 1u)) zero_action_row(env, a);  // wrappers.py:105-107
-    step_done(a, ctr);
+    step_done<VIEW>(a, ctr);
   }
   PROF_MARK(5);
   PROF_STORE;
@@ -752,6 +768,30 @@ VSS_API int vss_step_view(vss_handle h, int view, const float* policy_action, fl
     case VSS_VIEW_DMA: return launch_step<VSS_VIEW_DMA, false>(h, a, stream);
     default: return fail(VSS_E_INVALID, "vss_step_view: unknown view");
   }
+}
+
+VSS_API int vss_step_match(vss_handle h, const vss_match_team teams[2], float* action_buf, int64_t* reset_buf,
+                           float* obs, int64_t count_envs, int64_t n_matches, vss_match_board* board, void* stream) {
+  // everything that needs no handle first
+  if (!teams) return fail(VSS_E_INVALID, "vss_step_match: null argument");
+  for (int t = 0; t < 2; ++t) {
+    const int m = teams[t].mode;
+    if (m < VSS_TEAM_ZERO || m > VSS_TEAM_EXTERNAL) return fail(VSS_E_INVALID, "vss_step_match: unknown team mode");
+    if ((m == VSS_TEAM_SA || m == VSS_TEAM_CMA || m == VSS_TEAM_DMA) && !teams[t].policy_action)
+      return fail(VSS_E_INVALID, "vss_step_match: a policy team needs its policy action");
+  }
+  if (n_matches < 1) return fail(VSS_E_INVALID, "vss_step_match: n_matches must be >= 1");
+  if (!h || !action_buf || !reset_buf || !board) return fail(VSS_E_INVALID, "vss_step_match: null argument");
+  if (count_envs < 1 || count_envs > h->n) return fail(VSS_E_INVALID, "vss_step_match: count_envs outside [1, num_envs]");
+  if (h->range_count > 0) return fail(VSS_E_INVALID, "vss_step_match: whole-engine launches only (a step range is set)");
+  if (int rc = use_device(h)) return rc;
+  StepArgs a = base_args(h);
+  a.action_buf = action_buf; a.reset_buf = reinterpret_cast<long long*>(reset_buf); a.obs = obs;
+  for (int t = 0; t < 2; ++t) {
+    a.team_mode[t] = teams[t].mode; a.team_action[t] = teams[t].policy_action; a.team_rows[t] = teams[t].rows_bf16;
+  }
+  a.count_envs = count_envs; a.n_matches = n_matches; a.board = board;
+  return launch_step<VIEW_MATCH, false>(h, a, stream);
 }
 
 VSS_API int vss_step_view_host(vss_handle h, int view, const vss_view_buffers* dev, const float* policy_action_host,

@@ -164,6 +164,26 @@ class Engine:
             _ptr(ret_len, torch.int32, nv, "ret_len"), self._stream()))
 
 
+    def step_match(self, teams, action_buf, reset_buf, board, count_envs, n_matches, obs=None):
+        """`vss_step_match`: one step of a two-team match (include/vss_b200.h). teams = [(mode, policy_action or
+        None, rows_bf16 or None)] for blue and yellow; action_buf (N,2,3,2) f32 io; reset_buf (N) int64 io;
+        board = int64 tensor of _lib.BOARD_WORDS words (the vss_match_board, zeroed before the first step);
+        obs (N,2,3,52) f32 or None."""
+        n = self.num_envs
+        arr = (_lib.MatchTeam * 2)()
+        for k, (mode, act, rows) in enumerate(teams):
+            mode = int(mode)
+            nv = 3 * n if mode == _lib.TEAM_DMA else n
+            adim = 6 if mode == _lib.TEAM_CMA else 2
+            policy = mode in (_lib.TEAM_SA, _lib.TEAM_CMA, _lib.TEAM_DMA)
+            arr[k] = _lib.MatchTeam(mode, 0, _ptr(act, torch.float32, nv * adim, "policy_action") if policy else None,
+                                    _ptr(rows, torch.bfloat16, nv * 64, "rows_bf16") if policy else None)
+        check(self.lib.vss_step_match(
+            self._h, arr, _ptr(action_buf, torch.float32, n * 12, "action_buf"),
+            _ptr(reset_buf, torch.int64, n, "reset_buf"), _ptr(obs, torch.float32, n * 312, "obs"),
+            int(count_envs), int(n_matches), _ptr(board, torch.int64, _lib.BOARD_WORDS, "board"), self._stream()))
+
+
 def _engine_step_view_host(self, view, bufs, action_host, rows_host, num_ranges):
     """`vss_step_view_host`: pinned host action in, packed rows in pinned host memory out, pipelined over field
     ranges inside the library; returns when the rows are in host memory. `bufs`: _lib.ViewBuffers of device pointers."""
