@@ -313,6 +313,39 @@ typedef struct vss_match_board {
 VSS_API int vss_step_match(vss_handle h, const vss_match_team teams[2], float* action_buf, int64_t* reset_buf,
                            float* obs, int64_t count_envs, int64_t n_matches, vss_match_board* board, void* stream);
 
+/* ---- training against an opponent: a team in the yellow slots of the view step ----
+ * With an opponent set, every vss_step_view launch (whole-engine or a vss_set_step_range range) is one opponent view
+ * step. Restatement (what the tests check the kernels against):
+ *   1. action_buf = random_ou(action_buf) on all 12 slots (Philox stream 2 keyed by the device step index, as today);
+ *   2. the learner's slots = policy_action, exactly as the view does without an opponent;
+ *   3. the 6 yellow slots follow the opponent's mode (VSS_TEAM_*):
+ *        OU        keep the draw: no opponent; vss_step_view runs today's kernel
+ *        ZERO      draw x 0 (act[:] *= 0 on the drawn buffer: the sign of zero is kept)
+ *        SA        robot 0 = policy_action (N,2); robots 1-2 keep the draw
+ *        CMA / DMA the 6 slots = policy_action (N,6) / (3N,2)
+ *        EXTERNAL  the slots as the caller wrote them before the step (the noise is drawn, not stored there);
+ *   4. everything else is the view step: the buffer is stored un-clamped and clamped into the state; physics,
+ *      rewards, dones, the learner's outputs, episode statistics and aux outputs are unchanged; done rows of
+ *      action_buf are zeroed (all 12 slots);
+ *   5. after the masked reset, for every field: rows_bf16 = the opponent's policy input, the yellow rows (the
+ *      mirrored obs[:,1]) rounded to nearest even and padded to 64 columns, columns 52..63 never written: robot 0
+ *      -> row env (SA / CMA), robot i -> row 3 env + i (DMA); obs_f32 = the yellow team's (N,3,52) observation.
+ * Extra HBM bytes per field-step: policy action in 8 (SA) / 24 (CMA, DMA); bf16 rows out 104 (SA, CMA) / 312 (DMA);
+ * obs_f32 624 when requested. */
+typedef struct vss_view_opponent {
+  int32_t mode;               /* VSS_TEAM_*; OU = no opponent (today's kernel) */
+  int32_t reserved;
+  const float* policy_action; /* SA (N,2), CMA (N,6), DMA (3N,2); required by those modes */
+  void* rows_bf16;            /* SA/CMA (N,64), DMA (3N,64) bf16, or NULL */
+  float* obs_f32;             /* (N,3,52) yellow post-reset obs, or NULL */
+} vss_view_opponent;
+/* Sets (opp) or clears (NULL) the opponent of the following vss_step_view launches. Host-side state of the handle,
+ * like vss_set_step_aux: the struct is copied, its pointers are read when vss_step_view is called, so a captured
+ * graph records them. Arguments are checked before anything else (unknown mode, a policy mode without
+ * policy_action, then the handle). vss_step_view_host returns VSS_E_INVALID while an opponent is set; vss_step and
+ * vss_step_match ignore it. */
+VSS_API int vss_set_view_opponent(vss_handle h, const vss_view_opponent* opp);
+
 /* State access for parity tests and checkpointing: copies the SoA state
  * (VSS_STATE_WORDS x ld 32-bit words) device->device. */
 VSS_API int vss_get_state(vss_handle h, float* state_out, void* stream);

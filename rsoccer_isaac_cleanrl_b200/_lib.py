@@ -69,6 +69,13 @@ class MatchTeam(C.Structure):
     _fields_ = [("mode", C.c_int32), ("reserved", C.c_int32), ("policy_action", C.c_void_p), ("rows_bf16", C.c_void_p)]
 
 
+class ViewOpponent(C.Structure):
+    """`vss_view_opponent` of include/vss_b200.h."""
+
+    _fields_ = [("mode", C.c_int32), ("reserved", C.c_int32), ("policy_action", C.c_void_p), ("rows_bf16", C.c_void_p),
+                ("obs_f32", C.c_void_p)]
+
+
 # `vss_match_board` of include/vss_b200.h as int64 words: matches, length_sum, score_sum (float64 bits), steps,
 # frozen (low 32 bits)
 BOARD_WORDS = 5
@@ -111,6 +118,7 @@ _SYMBOLS = {
     "vss_step_fields_per_tile": (C.c_int, [_VP]),
     "vss_set_step_range": (C.c_int, [_VP, C.c_int64, C.c_int64]),
     "vss_step_match": (C.c_int, [_VP, C.POINTER(MatchTeam), _VP, _VP, _VP, C.c_int64, C.c_int64, _VP, _VP]),
+    "vss_set_view_opponent": (C.c_int, [_VP, C.POINTER(ViewOpponent)]),
     "vss_get_state": (C.c_int, [_VP, _VP, _VP]),
     "vss_set_state": (C.c_int, [_VP, _VP, _VP]),
     "vss_step_count": (C.c_uint64, [_VP]),

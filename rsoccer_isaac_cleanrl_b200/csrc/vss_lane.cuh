@@ -828,6 +828,11 @@ VSS_HD void st_bf16x4(void* base, long long off, const F4& v) {
 
 constexpr int VIEW_FULL = -1;
 constexpr int VIEW_MATCH = 3;  // vss_step_match: two teams, the scoreboard, no terminal observation / f32 rewards
+// VIEW_OPP + VSS_VIEW_*: the view step with an opponent in the yellow slots (vss_set_view_opponent). Everything the
+// view does is unchanged; the yellow slots follow the opponent's mode instead of the OU draw, and the yellow team's
+// post-reset observation is written for the opponent's next call.
+constexpr int VIEW_OPP = 8;
+VSS_HD constexpr int view_base(int view) { return view >= VIEW_OPP ? view - VIEW_OPP : view; }
 
 struct StepArgs {
   float* state; long long n, ld; unsigned long long goff;  // n = end of the field range of this launch
@@ -863,14 +868,20 @@ struct StepArgs {
   const float* team_action[2];
   void* team_rows[2];
   long long count_envs, n_matches;
-  vss_match_board* board;
+  // opponent views (VIEW_OPP + v) use team_mode / team_action / team_rows [1] for the yellow team and opp_obs for its
+  // (N,3,52) f32 post-reset observation (or null); sharing the board's word keeps the kernel parameters' layout
+  union {
+    vss_match_board* board;
+    float* opp_obs;
+  };
 };
 
 template <int VIEW>
 struct ViewShape {
-  static constexpr int F4_PER = (VIEW == VIEW_FULL || VIEW == VIEW_MATCH) ? F4_PER_FIELD
-                                                                          : (VIEW == VSS_VIEW_DMA ? 3 * F4_PER_ROW : F4_PER_ROW);
-  static constexpr int AGENTS = VIEW == VSS_VIEW_DMA ? 3 : 1;  // view "envs" per field
+  static constexpr int F4_PER = (VIEW == VIEW_FULL || VIEW == VIEW_MATCH)
+                                    ? F4_PER_FIELD
+                                    : (view_base(VIEW) == VSS_VIEW_DMA ? 3 * F4_PER_ROW : F4_PER_ROW);
+  static constexpr int AGENTS = view_base(VIEW) == VSS_VIEW_DMA ? 3 : 1;  // view "envs" per field
 };
 
 VSS_HD uint32_t step_index(const StepArgs& a) {
@@ -916,6 +927,19 @@ VSS_HD float match_slot(const StepArgs& a, long long env, int s, float prev, flo
   }
 }
 
+// Opponent view: yellow slot k (0..5) after the opponent's call (the restatement of vss_set_view_opponent), given
+// the value the caller left in the buffer and the slot's OU draw.
+VSS_HD float opp_slot(const StepArgs& a, long long env, int k, float prev, float ou) {
+  switch (a.team_mode[1]) {
+    case VSS_TEAM_ZERO: return fmul(ou, 0.0f);  // TeamZero on the drawn buffer: act[:] *= 0 keeps the sign of zero
+    case VSS_TEAM_SA: return k < 2 ? a.team_action[1][2 * env + k] : ou;
+    case VSS_TEAM_CMA:
+    case VSS_TEAM_DMA: return a.team_action[1][6 * env + k];  // (N,6) and (3N,2): the same 6 floats per field
+    case VSS_TEAM_EXTERNAL: return prev;                      // as the caller wrote it before the step
+    default: return ou;                                        // OU
+  }
+}
+
 // Phase 1a of a step for one field: state in, actions (+OU noise), progress restart, prev clones.
 template <int VIEW>
 VSS_HD void lane_phase1a(float* S, long long env, const StepArgs& a, const DevParams& P, const RngKey& key) {
@@ -943,12 +967,19 @@ VSS_HD void lane_phase1a(float* S, long long env, const StepArgs& a, const DevPa
 #pragma unroll
     for (int q = 0; q < 3; ++q) st4(ap + 4 * q, F4{act[4 * q], act[4 * q + 1], act[4 * q + 2], act[4 * q + 3]});
   } else if (VIEW != VIEW_FULL) {
+    float prev[6];  // (opponent views) the yellow slots as the caller left them
+#pragma unroll
+    for (int q = 0; q < 6; ++q) prev[q] = act[6 + q];
     ou_lane(act, P, key, step_index(a));  // action_buf = random_ou(action_buf)
-    if (VIEW == VSS_VIEW_SA) {     // act_view[:] = action
+    if (view_base(VIEW) == VSS_VIEW_SA) {     // act_view[:] = action
       act[0] = a.policy_action[2 * env]; act[1] = a.policy_action[2 * env + 1];
     } else {  // cma (N,6) and dma (3N,2): the same 6 contiguous floats per field
 #pragma unroll
       for (int q = 0; q < 6; ++q) act[q] = a.policy_action[6 * env + q];
+    }
+    if (VIEW >= VIEW_OPP) {  // the opponent's call on act[:, 1]
+#pragma unroll
+      for (int q = 0; q < 6; ++q) act[6 + q] = opp_slot(a, env, q, prev[q], act[6 + q]);
     }
     // the view keeps the un-clamped buffer (wrappers.py:102-103); done rows are zeroed in phase 5
     float* ap = a.action_buf + env * VSS_ACT_PER_FIELD;
@@ -997,10 +1028,16 @@ VSS_HD void actions_block(float* S, long long env, const StepArgs& a, const DevP
     st4(ab, F4{act[0], act[1], act[2], act[3]});
   } else if (VIEW != VIEW_FULL) {
     ou_block(act, P, key, step_index(a), (uint32_t)b);
-    if (VIEW == VSS_VIEW_SA) {
+    if (view_base(VIEW) == VSS_VIEW_SA) {
       if (b == 0) { act[0] = a.policy_action[2 * env]; act[1] = a.policy_action[2 * env + 1]; }
     } else {  // cma (N,6) and dma (3N,2): the same 6 contiguous floats per field
       for (int q = 4 * b; q < 6 && q < 4 * b + 4; ++q) act[q - 4 * b] = a.policy_action[6 * env + q];
+    }
+    if (VIEW >= VIEW_OPP) {  // the opponent's call on act[:, 1] (slots 6..11)
+      const float prev[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+      for (int q = 0; q < 4; ++q)
+        if (4 * b + q >= 6) act[q] = opp_slot(a, env, 4 * b + q - 6, prev[q], act[q]);
     }
     st4(ab, F4{act[0], act[1], act[2], act[3]});
   }
@@ -1146,7 +1183,7 @@ VSS_HD int lane_outputs(float* S, long long env, const StepArgs& a, const DevPar
       float r4[4];
 #pragma unroll
       for (int c = 0; c < 4; ++c) {
-        if (VIEW == VSS_VIEW_CMA) r4[c] = fdiv(fadd(fadd(rew[c], rew[4 + c]), rew[8 + c]), 3.0f);  // .mean(1)
+        if (view_base(VIEW) == VSS_VIEW_CMA) r4[c] = fdiv(fadd(fadd(rew[c], rew[4 + c]), rew[8 + c]), 3.0f);  // .mean(1)
         else r4[c] = rew[4 * j + c];
       }
       st4(a.rew + 4 * v, F4{r4[0], r4[1], r4[2], r4[3]});
@@ -1326,6 +1363,27 @@ VSS_HD void write_match_tile(const float* T, const uint32_t* tab, int lane, int 
     const F4 v = obs_gather(T, tab[j], e);
     if (a.obs) st4(a.obs + 4 * (env0 * F4_PER_FIELD + f), v);
     if (r >= 0) st_bf16x4(rows, r * 64 + (j - row * F4_PER_ROW) * 4, v);
+  }
+}
+
+// Opponent view: the yellow team's post-reset observation of the tile's fields (cooperative, all 32 lanes of `parts`
+// warps), gathered through obs-table entries 39..77 (the mirrored obs[:,1] rows): the f32 (N,3,52) rows when
+// a.opp_obs is set, and the policy opponent's bf16 rows (SA / CMA: robot 0 -> row env; DMA: robot i -> row 3 env + i).
+// Only robot 0 is gathered when nothing else goes anywhere.
+VSS_HD void write_opp_tile(const float* T, const uint32_t* tab, int lane, int valid, long long env0, const StepArgs& a,
+                           int part = 0, int parts = 1) {
+  const int m = a.team_mode[1];
+  void* rows = (m == VSS_TEAM_SA || m == VSS_TEAM_CMA || m == VSS_TEAM_DMA) ? a.team_rows[1] : nullptr;
+  if (!rows && !a.opp_obs) return;
+  constexpr int TEAM = 3 * F4_PER_ROW;
+  const int per = (a.opp_obs || m == VSS_TEAM_DMA) ? TEAM : F4_PER_ROW;
+  const int total = valid * per;
+  for (int f = lane + 32 * part; f < total; f += 32 * parts) {
+    const int e = f / per, j = f - e * per, i = j / F4_PER_ROW;
+    const F4 v = obs_gather(T, tab[TEAM + j], e);
+    if (a.opp_obs) st4(a.opp_obs + 4 * ((env0 + e) * TEAM + j), v);
+    const long long r = m == VSS_TEAM_DMA ? 3 * (env0 + e) + i : (i == 0 ? env0 + e : -1);
+    if (rows && r >= 0) st_bf16x4(rows, r * 64 + (j - i * F4_PER_ROW) * 4, v);
   }
 }
 

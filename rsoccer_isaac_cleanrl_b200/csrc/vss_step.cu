@@ -173,6 +173,7 @@ k_step(const __grid_constant__ StepArgs a, const __grid_constant__ DevParams P) 
   // 4. observation of the fields that were reset (vss.py:203)
   if (VIEW == VIEW_MATCH) write_match_tile(T, tab, lane, valid, env0, a);
   else write_obs_fields(T, tab, lane, PER_FIELD, ob, done_mask, obh, pk);
+  if (VIEW >= VIEW_OPP) write_opp_tile(T, tab, lane, valid, env0, a);  // the opponent's next input
   // 5. state out
   if (SYNC) __syncthreads();
   if (active) lane_phase5<VIEW>(S, env, a, code != LANE_RUNNING);
@@ -354,6 +355,7 @@ k_step_cta(const __grid_constant__ StepArgs a, const __grid_constant__ DevParams
   // 4. observation of the fields that were reset (vss.py:203); 5. state out
   if (VIEW == VIEW_MATCH) write_match_tile(T, tab, lane, valid, env0, a, warp, NW);
   else write_obs_fields(T, tab, lane, PER_FIELD, ob, done_mask, obh, pk, warp, NW);
+  if (VIEW >= VIEW_OPP) write_opp_tile(T, tab, lane, valid, env0, a, warp, NW);  // the opponent's next input
   if (active) store_state_words(S, a.state, a.ld, env, warp, NW);
   if (VIEW == VIEW_MATCH) {
     step_done<VIEW>(a, ctr);  // (done rows keep their actions: play_matches carries the OU state over)
@@ -490,6 +492,7 @@ struct vss_engine {
   int wpt_override;                                             // vss_set_step_warps_per_tile (0 = automatic)
   int fpt_override;                                             // vss_set_step_fields_per_tile (0 = automatic)
   int64_t range_first, range_count;                             // vss_set_step_range (count 0 = all fields)
+  vss_view_opponent opp;                                        // vss_set_view_opponent (mode OU = none)
   cudaStream_t host_stream[2];                                  // vss_step_view_host: the two pipeline streams ...
   cudaEvent_t host_start, host_done[2];                         // ... and their fork / join events (created on first use)
   bool host_ready;
@@ -654,6 +657,7 @@ VSS_API int vss_create(vss_handle* out, const vss_params* p, int64_t num_envs, i
   h->device = device; h->n = num_envs; h->ld = (num_envs + 31) / 32 * 32; h->goff = global_env_offset;
   h->aux_obs_bf16 = nullptr; h->aux_done_f = nullptr; h->aux_timeout_f = nullptr; h->packed_rows = nullptr;
   h->range_first = 0; h->range_count = 0; h->wpt_override = 0; h->fpt_override = 0; h->host_ready = false;
+  h->opp = vss_view_opponent{VSS_TEAM_OU, 0, nullptr, nullptr, nullptr};
   h->seed = seed; h->d_step = nullptr; h->params = *p; h->dp = derive_params(*p); h->state = nullptr;
   const size_t bytes = sizeof(float) * VSS_STATE_WORDS * (size_t)h->ld;
   e = cudaMalloc(&h->state, bytes);
@@ -762,6 +766,16 @@ VSS_API int vss_step_view(vss_handle h, int view, const float* policy_action, fl
   a.ep_ret = ep_ret; a.ep_len = ep_len; a.ret_ret = ret_ret; a.ret_len = ret_len;
   a.obs_bf16 = h->aux_obs_bf16; a.done_f = h->aux_done_f; a.timeout_f = h->aux_timeout_f;
   a.packed = h->packed_rows;
+  if (h->opp.mode != VSS_TEAM_OU) {  // the opponent variant of the view (today's kernel without one)
+    a.team_mode[1] = h->opp.mode; a.team_action[1] = h->opp.policy_action; a.team_rows[1] = h->opp.rows_bf16;
+    a.opp_obs = h->opp.obs_f32;
+    switch (view) {
+      case VSS_VIEW_SA: return launch_step<VIEW_OPP + VSS_VIEW_SA, false>(h, a, stream);
+      case VSS_VIEW_CMA: return launch_step<VIEW_OPP + VSS_VIEW_CMA, false>(h, a, stream);
+      case VSS_VIEW_DMA: return launch_step<VIEW_OPP + VSS_VIEW_DMA, false>(h, a, stream);
+      default: return fail(VSS_E_INVALID, "vss_step_view: unknown view");
+    }
+  }
   switch (view) {
     case VSS_VIEW_SA: return launch_step<VSS_VIEW_SA, false>(h, a, stream);
     case VSS_VIEW_CMA: return launch_step<VSS_VIEW_CMA, false>(h, a, stream);
@@ -799,6 +813,7 @@ VSS_API int vss_step_view_host(vss_handle h, int view, const vss_view_buffers* d
   if (!h || !dev || !policy_action_host || !rows_host || !dev->packed_rows || !dev->policy_action)
     return fail(VSS_E_INVALID, "vss_step_view_host: null argument");
   if (view != VSS_VIEW_SA && view != VSS_VIEW_CMA && view != VSS_VIEW_DMA) return fail(VSS_E_INVALID, "vss_step_view_host: unknown view");
+  if (h->opp.mode != VSS_TEAM_OU) return fail(VSS_E_INVALID, "vss_step_view_host: no opponents on the host-buffer path");
   if (int rc = use_device(h)) return rc;
   if (!h->host_ready) {
     for (int i = 0; i < 2; ++i) {
@@ -856,6 +871,18 @@ VSS_API int vss_step_view_host(vss_handle h, int view, const vss_view_buffers* d
 VSS_API int vss_set_step_aux(vss_handle h, void* obs_bf16, float* done_f32, float* timeout_f32) {
   if (!h) return fail(VSS_E_INVALID, "vss_set_step_aux: null handle");
   h->aux_obs_bf16 = obs_bf16; h->aux_done_f = done_f32; h->aux_timeout_f = timeout_f32;
+  return VSS_OK;
+}
+
+VSS_API int vss_set_view_opponent(vss_handle h, const vss_view_opponent* opp) {
+  if (opp) {  // everything that needs no handle first
+    const int m = opp->mode;
+    if (m < VSS_TEAM_ZERO || m > VSS_TEAM_EXTERNAL) return fail(VSS_E_INVALID, "vss_set_view_opponent: unknown team mode");
+    if ((m == VSS_TEAM_SA || m == VSS_TEAM_CMA || m == VSS_TEAM_DMA) && !opp->policy_action)
+      return fail(VSS_E_INVALID, "vss_set_view_opponent: a policy opponent needs its policy action");
+  }
+  if (!h) return fail(VSS_E_INVALID, "vss_set_view_opponent: null handle");
+  h->opp = opp ? *opp : vss_view_opponent{VSS_TEAM_OU, 0, nullptr, nullptr, nullptr};
   return VSS_OK;
 }
 

@@ -39,6 +39,7 @@ class Engine:
         self.ld = int(self.lib.vss_state_ld(self._h))
         self._aux_set = False
         self._packed_set = False
+        self._opp_set = False
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h.value:
@@ -130,14 +131,18 @@ class Engine:
 
     def step_view(self, view, policy_action, action_buf, reset_buf, obs_v, term_obs_v, rews_v, reward_v, done_v,
                   timeout_v, progress_v, ep_ret=None, ep_len=None, ret_ret=None, ret_len=None, obs_bf16=None,
-                  done_f=None, timeout_f=None, packed=None):
+                  done_f=None, timeout_f=None, packed=None, opponent=None):
         """`obs_bf16 (N',64) bf16`, `done_f (N') f32`, `timeout_f (N') f32`: optional side outputs
         (vss_set_step_aux) — the observation as the tensor-core MLP reads it, the flags as the GAE
         kernel reads them. `packed (N',112) uint8`: optional packed per-agent rows (vss_set_step_packed),
-        a CUDA tensor or a pinned host tensor (the kernel then stores across PCIe)."""
+        a CUDA tensor or a pinned host tensor (the kernel then stores across PCIe).
+        `opponent = (mode, policy_action or None, rows_bf16 or None, obs_f32 or None)`: the yellow team of this step
+        (vss_set_view_opponent); None or mode TEAM_OU = no opponent, today's view step."""
         n = self.num_envs
         nv = n * 3 if view == VIEW_DMA else n
         adim = 6 if view == VIEW_CMA else 2
+        if opponent is not None or self._opp_set:
+            self.set_view_opponent(opponent)
         if obs_bf16 is not None or done_f is not None or timeout_f is not None or self._aux_set:
             check(self.lib.vss_set_step_aux(self._h, _ptr(obs_bf16, torch.bfloat16, nv * 64, "obs_bf16"),
                                             _ptr(done_f, torch.float32, nv, "done_f"),
@@ -163,6 +168,23 @@ class Engine:
             _ptr(ep_len, torch.int32, nv, "ep_len"), _ptr(ret_ret, torch.float32, nv * 4, "ret_ret"),
             _ptr(ret_len, torch.int32, nv, "ret_len"), self._stream()))
 
+
+    def set_view_opponent(self, opponent):
+        """`vss_set_view_opponent`: opponent = (mode, policy_action, rows_bf16, obs_f32) as in step_view, or None."""
+        n = self.num_envs
+        if opponent is None or int(opponent[0]) == _lib.TEAM_OU:
+            check(self.lib.vss_set_view_opponent(self._h, None))
+            self._opp_set = False
+            return
+        mode, act, rows, obs = opponent
+        mode = int(mode)
+        ov = 3 * n if mode == _lib.TEAM_DMA else n
+        policy = mode in (_lib.TEAM_SA, _lib.TEAM_CMA, _lib.TEAM_DMA)
+        opp = _lib.ViewOpponent(
+            mode, 0, _ptr(act, torch.float32, ov * (6 if mode == _lib.TEAM_CMA else 2), "policy_action") if policy else None,
+            _ptr(rows, torch.bfloat16, ov * 64, "rows_bf16") if policy else None, _ptr(obs, torch.float32, n * 156, "obs_f32"))
+        check(self.lib.vss_set_view_opponent(self._h, C.byref(opp)))
+        self._opp_set = True
 
     def step_match(self, teams, action_buf, reset_buf, board, count_envs, n_matches, obs=None):
         """`vss_step_match`: one step of a two-team match (include/vss_b200.h). teams = [(mode, policy_action or

@@ -73,6 +73,7 @@ class _FusedView(Wrapper):
         self.returned_episode_returns = self.returned_episode_lengths = None
         self._host = None
         self._packed_out = None  # optional: where a step()'s packed rows go (vss_set_step_packed)
+        self.opponent = None     # set_opponent: the team in the yellow slots (None = OU noise, the reference's view)
 
     # ---- running episode statistics fused into the step epilogue (wrappers.py:50-87)
     def enable_episode_stats(self):
@@ -87,26 +88,51 @@ class _FusedView(Wrapper):
 
     def reset(self, **kwargs):
         observations = self.env.reset(**kwargs)
+        if self.opponent is not None:
+            self.opponent.load(observations["obs"])
         return {"obs": self._slice_obs(observations["obs"])}
 
+    def set_opponent(self, team, seed=0):
+        """Puts a team in the yellow slots of every following step: None (OU noise, the reference's view), a play.py
+        team object (TeamZero, TeamOU, TeamSA, TeamCMA, TeamDMA) or any `team(act, obs)` callable, which fills
+        act (N,3,2) in place from the yellow team's mirrored observation obs (N,3,52). Policy teams run on the
+        device (their actor, sampled with their own Philox stream from `seed`); see include/vss_b200.h,
+        vss_set_view_opponent, for what one step then computes. Call reset() afterwards: the opponent's first
+        input is the post-reset observation."""
+        from .. import _lib
+        from ..play import _team_mode
+        mode = _team_mode(team) if team is not None else _lib.TEAM_OU
+        self.opponent = None if mode == _lib.TEAM_OU else _Opponent(self, team, mode, seed)
+        if self.opponent is None:
+            self.task.engine.set_view_opponent(None)
+
     def step(self, action, obs_out=None, term_obs_out=None, reward_out=None, obs_bf16_out=None, done_f_out=None,
-             timeout_f_out=None):
+             timeout_f_out=None, opponent_issued=False):
         """One fused step. The optional `*_out` tensors (contiguous, right shape) make the kernel write
         the observation / terminal observation / scalar reward straight into caller storage — e.g. the
         `(T, N, …)` rollout slabs of the PPO loop (ppo…:258-272) — instead of the view's own buffers.
         `obs_bf16_out (N',64) bf16`, `done_f_out`, `timeout_f_out (N') f32` are extra copies in the form the
-        tensor-core MLP and the GAE kernel read (no conversion launches between the steps)."""
+        tensor-core MLP and the GAE kernel read (no conversion launches between the steps).
+        With an opponent (set_opponent) the step first runs the opponent's call (its actor launch, or the team
+        callable on its observation), then the kernel. `opponent_issued=True`: the caller has already issued the
+        device opponent's actor (`opponent.launch`) and advances its counter itself (the PPO rollout)."""
         task = self.task
         if action.device != task.device or action.dtype != torch.float32 or not action.is_contiguous():
             action = action.to(task.device, torch.float32).contiguous()
         obs = self._obs if obs_out is None else obs_out
         term_obs = self._term_obs if term_obs_out is None else term_obs_out
         reward = self._reward if reward_out is None else reward_out
+        opp = self.opponent
+        if opp is not None and not opponent_issued:
+            opp.act(self.action_buf)
         task.engine.step_view(self.VIEW, action, self.action_buf, task.reset_buf, obs, term_obs,
                               self._rews, reward, self._done, self._timeout_u8, self._progress,
                               self.episode_returns, self.episode_lengths, self.returned_episode_returns,
                               self.returned_episode_lengths, obs_bf16=obs_bf16_out, done_f=done_f_out,
-                              timeout_f=timeout_f_out, packed=self._packed_out)
+                              timeout_f=timeout_f_out, packed=self._packed_out,
+                              opponent=None if opp is None else opp.spec)
+        if opp is not None and not opponent_issued and opp.device is not None:
+            opp.device.counter.add_(1)
         task._obs_stale = True
         infos = task.extras
         infos["rews"] = self._rews
@@ -160,6 +186,8 @@ class _FusedView(Wrapper):
         own H2D copy -> kernel (-> D2H copy) on one of two side streams. Same kernels, same RNG keys: the
         device-side results are bit-identical to `step()`."""
         task, nv = self.task, self.num_view_envs
+        if self.opponent is not None:
+            raise NotImplementedError("step_host: opponents run on the device path only (step())")
         packed = obs_dtype == torch.bfloat16
         if not packed and obs_dtype != torch.float32:
             raise ValueError("step_host: obs_dtype must be torch.bfloat16 or torch.float32")
@@ -245,6 +273,62 @@ class _FusedView(Wrapper):
     @property
     def d2h_bytes_per_step(self):
         return self.d2h_bytes(torch.bfloat16)
+
+
+class _Opponent:
+    """The yellow team of a fused view (set_opponent): its device mode and the buffers the step kernel reads and
+    writes for it. `spec` is the `opponent` argument of Engine.step_view.
+      policy teams, tc backend  play._DevicePolicy: bf16 actor weights, its own Philox seed / counter, its bf16 rows
+                                (written by the step kernel) and the action of one fused actor launch (`launch`);
+      policy teams, fp32 Agent  (mlp_backend "torch") the Agent's sampled action on the f32 observation, passed in
+                                the same SA / CMA / DMA mode (the OU slots still come from the kernel);
+      EXTERNAL                  the callable, run on the f32 observation before the step;
+      ZERO                      nothing."""
+
+    def __init__(self, view, team, mode, seed):
+        from .. import _lib
+        from ..play import _DevicePolicy, _team_seed
+        task = view.task
+        n, dev = task.num_fields, task.device
+        self.team, self.mode = team, mode
+        self.device = None
+        self.obs_f32 = None
+        policy = mode in (_lib.TEAM_SA, _lib.TEAM_CMA, _lib.TEAM_DMA)
+        if policy and getattr(team.agent, "mlp_backend", "tc") == "tc":
+            self.device = _DevicePolicy(team, mode, 1, task.obs_buf.view(n * 6, -1), n, _team_seed(seed, 1))
+            self.spec = (mode, self.device.action, self.device.rows, None)
+            return
+        self.obs_f32 = torch.zeros((n, 3, task.num_obs), device=dev, dtype=torch.float32)
+        self.obs_f32.copy_(task.obs_buf[:, 1])
+        if policy:
+            self.action = torch.zeros((3 * n, 2) if mode == _lib.TEAM_DMA else (n, 6 if mode == _lib.TEAM_CMA else 2),
+                                      device=dev, dtype=torch.float32)
+            self.spec = (mode, self.action, None, self.obs_f32)
+        else:
+            self.spec = (mode, None, None, self.obs_f32 if mode == _lib.TEAM_EXTERNAL else None)
+
+    def load(self, full_obs):
+        """The opponent's input from a full (N,2,3,52) post-reset observation: obs[:, 1]."""
+        if self.device is not None:
+            self.device.load_rows(full_obs.reshape(-1, full_obs.shape[-1]))
+        if self.obs_f32 is not None:
+            self.obs_f32.copy_(full_obs[:, 1])
+
+    def launch(self, call_offset=0):
+        """The device opponent's fused actor launch (sampling call index = counter + call_offset)."""
+        self.device.launch(call_offset)
+
+    def act(self, action_buf):
+        """The opponent's call before a step."""
+        from .. import _lib
+        if self.device is not None:
+            self.launch(0)
+        elif self.mode == _lib.TEAM_EXTERNAL:
+            self.team(action_buf[:, 1], self.obs_f32)
+        elif self.mode in (_lib.TEAM_SA, _lib.TEAM_CMA, _lib.TEAM_DMA):
+            x = self.obs_f32.view(-1, self.obs_f32.shape[-1]) if self.mode == _lib.TEAM_DMA else self.obs_f32[:, 0]
+            with torch.no_grad():
+                self.action.copy_(self.team.agent.get_action_and_value(x.contiguous())[0].view(self.action.shape))
 
 
 class SingleAgent(_FusedView):

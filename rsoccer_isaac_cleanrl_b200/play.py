@@ -52,6 +52,13 @@ class TeamAgent(Team):
         self.agent.load_state_dict(torch.load(path, map_location=device))  # reference state_dict keys
         self.agent.eval()
 
+    @classmethod
+    def from_agent(cls, agent):
+        """The team of an Agent already in memory (a self-play snapshot, for instance): no checkpoint is read."""
+        team = cls.__new__(cls)
+        team.agent = agent
+        return team
+
 
 class TeamSA(TeamAgent):
     """A single-agent policy drives robot 0; robots 1-2 follow OU noise (play.py:51-54)."""
@@ -166,12 +173,17 @@ class _DevicePolicy:
         robots = 3 if mode == _lib.TEAM_DMA else 1
         nv = n * robots
         # the team's rows of the observation: (field, team, robot) -> row 6 field + 3 team + robot of obs (N*6, 52)
-        idx = (6 * torch.arange(n, device=dev)[:, None] + 3 * side + torch.arange(robots, device=dev)[None]).reshape(-1)
-        self.rows = gather_pad_bf16(obs_flat, idx, 64)
+        self._idx = (6 * torch.arange(n, device=dev)[:, None] + 3 * side + torch.arange(robots, device=dev)[None]).reshape(-1)
+        self.rows = gather_pad_bf16(obs_flat, self._idx, 64)
         self.action = torch.zeros((nv, 6 if mode == _lib.TEAM_CMA else 2), device=dev, dtype=torch.float32)
         self.logprob = torch.empty(nv, device=dev, dtype=torch.float32)
         self.counter = torch.zeros(1, device=dev, dtype=torch.int32)
         self.seed = seed
+
+    def load_rows(self, obs_flat):
+        """Re-gathers the team's rows from a full (N*6, 52) observation (after a reset), into the same buffer."""
+        from .engine import gather_pad_bf16
+        self.rows.copy_(gather_pad_bf16(obs_flat, self._idx, 64))
 
     def launch(self, call_offset):
         from .engine import mlp_forward_fused

@@ -82,6 +82,11 @@ def parse_args(argv=None):
     p.add_argument("--grad-allreduce", type=str, default="auto", choices=["auto", "peer", "nccl"],
                    help="multi-GPU gradient sum: peer = one hand-written kernel per rank over NVLink peer memory "
                         "(CUDA IPC, one node); nccl = torch.distributed.all_reduce; auto = peer when it can be set up")
+    p.add_argument("--opponent", type=str, default="ou",
+                   help="the yellow team during training: ou (OU noise, the reference), zero, self (a frozen snapshot "
+                        "of the learner) or ppo-sa|ppo-sa-x3|ppo-cma|ppo-dma:PATH (a checkpoint)")
+    p.add_argument("--opponent-refresh", type=int, default=10,
+                   help="--opponent self: the snapshot is taken before update 1 and then every K updates")
     p.add_argument("--quiet", type=b, default=False, nargs="?", const=True)
     p.add_argument("--tensorboard", type=b, default=True, nargs="?", const=True,
                    help="write the reference's scalar tags (losses/*, Charts/SPS, rws/episodic_*) with SummaryWriter")
@@ -309,6 +314,27 @@ def _make_writer(args, rank, log):
     return writer
 
 
+_SELF_TEAM = {"sa": "TeamSA", "cma": "TeamCMA", "dma": "TeamDMA"}
+
+
+def make_opponent(args, agent, envs, device, backend):
+    """(team, frozen Agent or None) for --opponent; team None = OU noise (the reference's view, today's kernel)."""
+    from . import play
+    spec = getattr(args, "opponent", "ou")
+    if spec == "ou":
+        return None, None
+    if spec == "self":  # a frozen copy of the learner's actor, in the learner's own mode
+        frozen = Agent(envs, mlp_backend=backend).to(device)
+        frozen.load_state_dict(agent.state_dict())
+        frozen.requires_grad_(False)
+        frozen.eval()
+        return getattr(play, _SELF_TEAM[args.env_id]).from_agent(frozen), frozen
+    algo, _, path = spec.partition(":")
+    if algo not in ("zero", "ppo-sa", "ppo-sa-x3", "ppo-cma", "ppo-dma") or (algo != "zero" and not path):
+        raise ValueError(f"--opponent: expected ou, zero, self or ALGO:PATH, got {spec!r}")
+    return play.get_team(algo, path or None, str(device), backend), None
+
+
 def train(args, log=print, hook=None):
     import torch.distributed as dist
     from .envs import RecordEpisodeStatisticsTorch, make_env
@@ -324,6 +350,7 @@ def train(args, log=print, hook=None):
 
     writer = _make_writer(args, rank, log)
     unwrapped_env, envs = make_env(args)
+    view = envs
     envs = ExtractObsWrapper(envs)
     envs = RecordEpisodeStatisticsTorch(envs, device)
     envs.single_action_space = envs.action_space
@@ -355,6 +382,24 @@ def train(args, log=print, hook=None):
     grad_sum = flat_grad if peer_grads is None else torch.zeros_like(flat)
     optimizer = FlatAdam(flat, grad_sum, lr=args.learning_rate, eps=1e-5)
 
+    # the yellow team (--opponent): its own Philox stream per rank, like the learner's sampling stream
+    opp_team, opp_frozen = make_opponent(args, agent, envs, device, backend)
+    opp = opp_dev = None
+    if opp_team is not None:
+        from .play import _team_seed
+        view.set_opponent(opp_team, seed=_team_seed(args.seed + 7919 * (rank + 1), 1))
+        opp = view.opponent
+        opp_dev = opp.device if opp is not None else None   # a policy opponent whose actor runs on the device
+
+    def opponent_snapshot(update):
+        """--opponent self: copy the learner's weights into the frozen Agent's static fp32 buffers and their bf16
+        copies, outside any graph: later rollout replays read the new snapshot."""
+        with torch.no_grad():
+            for p_o, p_l in zip(opp_frozen.parameters(), agent.parameters()):
+                p_o.copy_(p_l)
+            if opp_dev is not None:
+                opp_dev.mw.refresh()
+
     T, N = args.num_steps, args.num_envs
     oshape, ashape = envs.single_observation_space.shape, envs.single_action_space.shape
     z = lambda *s: torch.zeros(s, dtype=torch.float32, device=device)
@@ -376,6 +421,8 @@ def train(args, log=print, hook=None):
         # the critic runs beside the actor on a second stream (fork/join inside the captured graphs): at
         # 4096 rows one network's GEMMs fill less than half of the SMs
         side = torch.cuda.Stream(device=device)
+        # the opponent's actor runs beside the learner's forward on a stream of its own
+        opp_stream = torch.cuda.Stream(device=device) if opp_dev is not None else None
 
     def on_side(fn):
         """Run fn() on the side stream, ordered after everything queued so far on the current one.
@@ -419,6 +466,10 @@ def train(args, log=print, hook=None):
                 # actor mean + action sample + log-prob (and the critic's value) in ONE launch (csrc/mlp_fused.cu); the
                 # sampling stream's call index is counter + step, the counter advances by T once per rollout
                 x16 = x16_buf[step & 1]
+                if opp_dev is not None:  # its rows were written by the previous env step; its action is read by this one
+                    opp_stream.wait_stream(torch.cuda.current_stream(device))
+                    with torch.cuda.stream(opp_stream):
+                        opp_dev.launch(step)
                 samp = dict(logstd=logstd_flat, counter=sample_ctr, seed=sample_seed, call_offset=step,
                             action=actions[step], logprob=logprobs[step])
                 if one_launch:
@@ -426,12 +477,17 @@ def train(args, log=print, hook=None):
                 else:
                     on_side(lambda: mlp_forward_fused(x16, [nets[1] + (values[step],)]))
                     mlp_forward_fused(x16, [nets[0] + (False,)], sampling=samp)
+                if opp_dev is not None:
+                    torch.cuda.current_stream(device).wait_stream(opp_stream)
                 envs.step(actions[step], obs_out=obs_all[step + 1], term_obs_out=term_obs_all[step],
                           reward_out=rewards[step], obs_bf16_out=x16_buf[(step + 1) & 1],
-                          done_f_out=next_dones[step], timeout_f_out=next_timeouts[step])
+                          done_f_out=next_dones[step], timeout_f_out=next_timeouts[step],
+                          opponent_issued=opp_dev is not None)
                 if not one_launch:
                     join_side()
             sample_ctr.add_(T)
+            if opp_dev is not None:
+                opp_dev.counter.add_(T)
             # V(terminal observation) (ppo…:272). Where the step did not end an episode the terminal observation IS the
             # next observation (the step kernel writes both from the same registers), so its value is the next step's
             # critic output, bit for bit (every row of the fused forward is computed independently of its neighbours):
@@ -620,6 +676,10 @@ def train(args, log=print, hook=None):
     t_roll = t_upd = 0.0
     for update in range(1, num_updates + 1):
         state["update"] = update
+        if opp_frozen is not None and (update - 1) % max(1, args.opponent_refresh) == 0:
+            opponent_snapshot(update)
+            if writer is not None:
+                writer.add_scalar("opponent/snapshot_update", update, global_step)
         if args.anneal_lr:
             optimizer.param_groups[0]["lr"] = anneal_lr(update, num_updates, args.learning_rate)
         tr0 = time.time()
@@ -653,7 +713,7 @@ def train(args, log=print, hook=None):
             hook(update, dict(obs=obs_all, actions=actions, logprobs=logprobs, rewards=rewards, values=values,
                               next_values=next_values, advantages=advantages, returns=returns, flat=flat,
                               flat_grad=flat_grad, term_obs=term_obs_all, next_dones=next_dones,
-                              agent=agent, env=unwrapped_env, stats=mb_stats))
+                              agent=agent, env=unwrapped_env, stats=mb_stats, opponent=opp))
         stats["rollout_wall"].append(tu0 - tr0)
         stats["update_wall"].append(time.time() - tu0)
         sps = int(global_step / (time.time() - start_time))
@@ -703,6 +763,7 @@ def train(args, log=print, hook=None):
         peer_grads.close()
     stats["agent"] = agent
     stats["env"] = unwrapped_env
+    stats["opponent"] = opp
     return stats
 
 
