@@ -383,7 +383,10 @@ VSS_API int vss_gae(const float* rewards, const float* values, const float* next
  *                 dW = dZ^T X with the batch as K; no transposed copies needed).
  *   epilogue: 0 out_bf16 = tanh(acc + bias[n]); 1 out_bf16 = acc * (1 - aux[m,n]^2) (aux bf16);
  *             2 out_f32 += acc (atomic, split-K; caller zeroes out); 3 out_f32 = acc + bias[n].
- *   lda/ldb/ldo/ld_aux in elements; K multiple of 64 (K-major), N multiple of 64. */
+ *   lda/ldb/ldo/ld_aux in elements; K multiple of 64 (K-major), N multiple of 64. lda/ldb: multiples of 8, at least
+ *   the row they hold (K; M/N with mn_major). ldo >= N, a multiple of 8 for bf16 outputs and of 4 for epilogue 3;
+ *   out (epilogues 0, 1, 3) and bias 16-byte aligned; epilogue 1: ld_aux >= N, a multiple of 8, aux 16-byte
+ *   aligned. Other layouts return VSS_E_INVALID before any CUDA call. */
 VSS_API int vss_gemm_bf16_tn(const void* A, int lda, const void* B, int ldb, void* out, int ldo, int M,
                              int N, int K, int epilogue, const float* bias, const void* aux, int ld_aux,
                              int splits, int mn_major, void* stream);
@@ -393,17 +396,20 @@ VSS_API int vss_gemm_bf16_tn_colsum(const void* A, int lda, const void* B, int l
                                     int N, int K, int epilogue, const float* bias, const void* aux, int ld_aux,
                                     int splits, int mn_major, float* colsum, void* stream);
 VSS_API const char* vss_gemm_last_error(void);
-/* out[N] (f32) += column sums of the bf16 matrix x [M,N] (row stride ld): bias gradients. */
+/* out[N] (f32) += column sums of the bf16 matrix x [M,N] (row stride ld): bias gradients. N and ld even, ld >= N,
+ * x 4-byte aligned. */
 VSS_API int vss_colsum_bf16(const void* x, int ld, int M, int N, float* out, void* stream);
 /* dst [M,ncol_pad] bf16 = zero-padded src[idx[m] (or m if idx is NULL), :ncol] f32: the minibatch
- * gather b_obs[mb_inds] (ppo...:314) fused with the bf16 conversion and K padding. */
+ * gather b_obs[mb_inds] (ppo...:314) fused with the bf16 conversion and K padding. ncol_pad even, dst 4-byte
+ * aligned. */
 VSS_API int vss_gather_pad_bf16(const float* src, const int64_t* idx, int M, int ncol, int ncol_pad, void* dst,
                                 void* stream);
 
 /* Output head of the Agent MLPs (Linear 256 -> n_out in {1,2,6}, ppo...:138,151) and its backward
  * fused with tanh' of the last hidden layer: dz = (dout W) * (1 - h^2) (bf16), dW += dout^T h,
  * db += sum dout; dz_colsum [256] += column sums of dz (bias gradient of the last hidden layer) when
- * not NULL. h [M,256] bf16, W [n_out,256] f32, out/dout [M,n_out] f32. */
+ * not NULL. h [M,256] bf16, W [n_out,256] f32, out/dout [M,n_out] f32. ldh/ldz >= 256 and multiples of 8, h and dz
+ * 16-byte aligned. */
 VSS_API int vss_head_forward(const void* h, int ldh, const float* W, const float* b, float* out, int M, int n_out,
                              void* stream);
 VSS_API int vss_head_backward(const float* dout, const void* h, int ldh, const float* W, void* dz, int ldz,

@@ -833,7 +833,7 @@ VSS_API const char* vss_gemm_last_error(void) { return g_tc_error.c_str(); }
 //   mn_major = 0: A is [M,K], B is [N,K] row-major (K contiguous) — forward and dgrad.
 //   mn_major = 1: A is [K,M], B is [K,N] row-major (the reduction index is the row) — wgrad
 //                 dW[N_out,K_in] = sum_batch dZ[batch,N_out] * X[batch,K_in], no transposes needed.
-// lda/ldb in elements (multiples of 8). K: multiple of 64, or ragged with mn_major (TMA zero-fills
+// lda/ldb/ldo/ld_aux in elements (layout rules: include/vss_b200.h). K: multiple of 64, or ragged with mn_major (TMA zero-fills
 // rows past K). N multiple of 64. epilogue: see tc::Epilogue. splits > 1 only with EPI_ATOMIC_F32
 // (the caller zeroes `out`). Returns 0 or a negative VSS_E_* code (message: vss_gemm_last_error).
 VSS_API int vss_gemm_bf16_tn(const void* A, int lda, const void* B, int ldb, void* out, int ldo, int M, int N, int K,
@@ -854,14 +854,36 @@ VSS_API int vss_gemm_bf16_tn_colsum(const void* A, int lda, const void* B, int l
     return VSS_E_INVALID;
   }
   if (!A || !B || !out || M <= 0 || N <= 0 || K <= 0) { g_tc_error = "vss_gemm_bf16_tn: bad argument"; return VSS_E_INVALID; }
+  if (epilogue < EPI_BIAS_TANH_BF16 || epilogue > EPI_BIAS_F32 || (mn_major && epilogue != EPI_ATOMIC_F32)) {
+    g_tc_error = "vss_gemm_bf16_tn: unsupported epilogue / layout combination"; return VSS_E_INVALID;
+  }
   if ((!mn_major && K % BK != 0) || N % 64 != 0 || lda % 8 != 0 || ldb % 8 != 0 || (mn_major && M % 128 != 0)) {
     g_tc_error = "vss_gemm_bf16_tn: K must be a multiple of 64 (K-major), N of 64, lda/ldb of 8, M of 128 (MN-major)";
     return VSS_E_INVALID;
+  }
+  if (lda < (mn_major ? M : K) || ldb < (mn_major ? N : K)) {
+    g_tc_error = "vss_gemm_bf16_tn: lda/ldb smaller than the rows of A/B"; return VSS_E_INVALID;
+  }
+  // The epilogues store bf16 rows as 16-byte pieces and f32 rows (EPI_BIAS_F32) as float4, read the bias as float4
+  // and the tanh' operand as 16-byte pieces: every row start they touch must be 16-byte aligned. The atomic epilogue
+  // falls back to scalar reductions on unaligned addresses (red_add_v4).
+  const bool bf16_out = epilogue == EPI_BIAS_TANH_BF16 || epilogue == EPI_DTANH_BF16;
+  if (ldo < N || (bf16_out && ldo % 8 != 0) || (epilogue == EPI_BIAS_F32 && ldo % 4 != 0) ||
+      (epilogue != EPI_ATOMIC_F32 && reinterpret_cast<uintptr_t>(out) % 16 != 0)) {
+    g_tc_error = "vss_gemm_bf16_tn: ldo must be >= N (a multiple of 8 for bf16 outputs, of 4 for EPI_BIAS_F32) and out "
+                 "16-byte aligned";
+    return VSS_E_INVALID;
+  }
+  if (bias && reinterpret_cast<uintptr_t>(bias) % 16 != 0) {
+    g_tc_error = "vss_gemm_bf16_tn: bias must be 16-byte aligned"; return VSS_E_INVALID;
   }
   if (splits < 1) splits = 1;
   if (splits > 1 && epilogue != EPI_ATOMIC_F32) { g_tc_error = "vss_gemm_bf16_tn: split-K needs the atomic epilogue"; return VSS_E_INVALID; }
   if ((epilogue == EPI_BIAS_TANH_BF16 && !bias) || (epilogue == EPI_DTANH_BF16 && !aux)) {
     g_tc_error = "vss_gemm_bf16_tn: missing bias/aux"; return VSS_E_INVALID;
+  }
+  if (epilogue == EPI_DTANH_BF16 && (ld_aux < N || ld_aux % 8 != 0 || reinterpret_cast<uintptr_t>(aux) % 16 != 0)) {
+    g_tc_error = "vss_gemm_bf16_tn: ld_aux must be >= N and a multiple of 8, aux 16-byte aligned"; return VSS_E_INVALID;
   }
   // tile width of the one-CTA kernel: 128 x 256 for the split-K wgrad shapes that do not reach the CTA-pair kernel
   // (short reductions), else 128 x 128 / 128 x 64
@@ -886,7 +908,7 @@ VSS_API int vss_gemm_bf16_tn_colsum(const void* A, int lda, const void* B, int l
   cudaError_t e = cudaSuccess;
   // forward and dgrad with N a multiple of 256 and enough row tiles: the CTA-pair kernel (tcgen05 cta_group::2)
   if ((epilogue == EPI_BIAS_TANH_BF16 || epilogue == EPI_DTANH_BF16) && !mn_major && splits == 1 && N % 256 == 0 &&
-      N <= 512 && M >= 256 * 74 && (epilogue != EPI_DTANH_BF16 || ld_aux % 8 == 0)) {
+      N <= 512 && M >= 256 * 74) {
     // A: 128-row boxes; B: 128-row boxes (this CTA's half of the 256 columns); out / tanh' operand: 32 x 64 boxes
     CUtensorMap ma2, mb2, mo2, mx2;
     bool ok2 = make_map(&ma2, A, M, K, lda, BM) && make_map(&mb2, B, N, K, ldb, 128) && make_map(&mo2, out, M, N, ldo, 32);
@@ -918,6 +940,9 @@ VSS_API int vss_gemm_bf16_tn_colsum(const void* A, int lda, const void* B, int l
 // out[N] (f32) += column sums of x [M,N] bf16 (row stride ld elements). N even.
 VSS_API int vss_colsum_bf16(const void* x, int ld, int M, int N, float* out, void* stream) {
   if (!x || !out || M <= 0 || N <= 0 || (N & 1)) { g_tc_error = "vss_colsum_bf16: bad argument"; return VSS_E_INVALID; }
+  if (ld < N || (ld & 1) || reinterpret_cast<uintptr_t>(x) % 4 != 0) {  // rows are read as bf16 pairs
+    g_tc_error = "vss_colsum_bf16: ld must be even and >= N, x 4-byte aligned"; return VSS_E_INVALID;
+  }
   const int col_blocks = (N + 63) / 64;
   int row_blocks = (148 * 8 + col_blocks - 1) / col_blocks;
   int rows_per_block = (M + row_blocks - 1) / row_blocks;
@@ -936,6 +961,9 @@ VSS_API int vss_gather_pad_bf16(const float* src, const int64_t* idx, int M, int
   if (!src || !dst || M <= 0 || ncol <= 0 || ncol_pad < ncol || (ncol_pad & 1)) {
     g_tc_error = "vss_gather_pad_bf16: bad argument"; return VSS_E_INVALID;
   }
+  if (reinterpret_cast<uintptr_t>(dst) % 4 != 0) {  // written as bf16 pairs
+    g_tc_error = "vss_gather_pad_bf16: dst must be 4-byte aligned"; return VSS_E_INVALID;
+  }
   const long long total = (long long)M * (ncol_pad / 2);
   tc::k_gather_pad_bf16<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
       src, reinterpret_cast<const long long*>(idx), M, ncol, ncol_pad, reinterpret_cast<__nv_bfloat16*>(dst));
@@ -948,6 +976,9 @@ VSS_API int vss_gather_pad_bf16(const float* src, const int64_t* idx, int M, int
 VSS_API int vss_head_forward(const void* h, int ldh, const float* W, const float* b, float* out, int M, int n_out,
                              void* stream) {
   if (!h || !W || !b || !out || M <= 0) { g_tc_error = "vss_head_forward: bad argument"; return VSS_E_INVALID; }
+  if (ldh < 256 || ldh % 8 != 0 || reinterpret_cast<uintptr_t>(h) % 16 != 0) {  // rows are read as 16-byte pieces
+    g_tc_error = "vss_head_forward: ldh must be >= 256 and a multiple of 8, h 16-byte aligned"; return VSS_E_INVALID;
+  }
   const __nv_bfloat16* hp = reinterpret_cast<const __nv_bfloat16*>(h);
   const int blocks = std::min((M + 7) / 8, 148 * 8);
   cudaStream_t st = (cudaStream_t)stream;
@@ -965,6 +996,11 @@ VSS_API int vss_head_forward(const void* h, int ldh, const float* W, const float
 VSS_API int vss_head_backward(const float* dout, const void* h, int ldh, const float* W, void* dz, int ldz, float* dW,
                               float* db, float* dz_colsum, int M, int n_out, void* stream) {
   if (!dout || !h || !W || !dz || !dW || !db || M <= 0) { g_tc_error = "vss_head_backward: bad argument"; return VSS_E_INVALID; }
+  if (ldh < 256 || ldh % 8 != 0 || ldz < 256 || ldz % 8 != 0 || reinterpret_cast<uintptr_t>(h) % 16 != 0 ||
+      reinterpret_cast<uintptr_t>(dz) % 16 != 0) {  // h rows are read and dz rows written as 16-byte pieces
+    g_tc_error = "vss_head_backward: ldh/ldz must be >= 256 and multiples of 8, h and dz 16-byte aligned";
+    return VSS_E_INVALID;
+  }
   const __nv_bfloat16* hp = reinterpret_cast<const __nv_bfloat16*>(h);
   __nv_bfloat16* zp = reinterpret_cast<__nv_bfloat16*>(dz);
   // resident blocks per SM: 3 (n_out <= 2, <= 85 registers) or 1 (n_out = 6, 162 registers): one wave, more rows in flight
