@@ -884,6 +884,24 @@ struct ViewShape {
   static constexpr int AGENTS = view_base(VIEW) == VSS_VIEW_DMA ? 3 : 1;  // view "envs" per field
 };
 
+// The output rows of the tile whose first field is env0: observation, terminal observation (or null) and, for the
+// views only, the same rows as bf16 padded to 64 columns and the packed rows (each or null).
+struct TileOut { float* ob; float* tob; void* obh; void* pk; };
+template <int VIEW>
+VSS_HD TileOut tile_out(const StepArgs& a, long long env0) {
+  constexpr int PER_FIELD = ViewShape<VIEW>::F4_PER, AGENTS = ViewShape<VIEW>::AGENTS;
+  TileOut o;
+  o.ob = a.obs + env0 * (PER_FIELD * 4);
+  o.tob = a.term_obs ? a.term_obs + env0 * (PER_FIELD * 4) : nullptr;
+  o.obh = (VIEW != VIEW_FULL && a.obs_bf16)
+              ? static_cast<void*>(static_cast<unsigned short*>(a.obs_bf16) + env0 * (AGENTS * 64))
+              : nullptr;
+  o.pk = (VIEW != VIEW_FULL && a.packed)
+             ? static_cast<void*>(static_cast<char*>(a.packed) + env0 * (AGENTS * VSS_PACKED_ROW_BYTES))
+             : nullptr;
+  return o;
+}
+
 VSS_HD uint32_t step_index(const StepArgs& a) {
 #if defined(__CUDA_ARCH__)
   return (uint32_t)__ldcg(a.step_ctr);  // read at L2, where the advancing CTA's add lands
@@ -908,35 +926,52 @@ VSS_HD void store_state(const float* S, float* state, long long ld, long long en
   for (int w = 0; w < VSS_STATE_WORDS; ++w) dst[(long long)w * ld] = S[w * LDS];
 }
 
-// Match mode: does either team draw OU noise (TeamOU, and robots 1-2 of TeamSA)?
-VSS_HD bool match_needs_ou(const StepArgs& a) {
+// Does the step draw OU noise? The views do; a match does if a team needs it (TeamOU, and robots 1-2 of TeamSA).
+template <int VIEW>
+VSS_HD bool draws_ou(const StepArgs& a) {
+  if (VIEW != VIEW_MATCH) return VIEW != VIEW_FULL;
   return a.team_mode[0] == VSS_TEAM_OU || a.team_mode[0] == VSS_TEAM_SA || a.team_mode[1] == VSS_TEAM_OU ||
          a.team_mode[1] == VSS_TEAM_SA;
 }
-// Match mode: action slot s (0..11) of the field after its team's call (play.py:34-64), given the buffer's previous
-// value and the OU draw of the slot.
-VSS_HD float match_slot(const StepArgs& a, long long env, int s, float prev, float ou) {
-  const int t = s >= 6 ? 1 : 0, k = s - 6 * t;
-  switch (a.team_mode[t]) {
-    case VSS_TEAM_ZERO: return fmul(prev, 0.0f);  // act[:] *= 0 keeps the sign of zero
-    case VSS_TEAM_OU: return ou;
-    case VSS_TEAM_SA: return k < 2 ? a.team_action[t][2 * env + k] : ou;
+// Action slot k (0..5) of a team after its call (play.py:34-64), from the team's mode and policy action (SA (N,2),
+// CMA (N,6), DMA (3N,2): the same 6 floats per field). `found` is the buffer as the team finds it (the previous value
+// in a match, the OU draw in a view), `prev` the value the caller wrote, `ou` the slot's OU draw. The C-ABI entries
+// accept only the VSS_TEAM_* modes.
+VSS_HD float team_slot(int mode, const float* action, long long env, int k, float found, float prev, float ou) {
+  switch (mode) {
+    case VSS_TEAM_ZERO: return fmul(found, 0.0f);  // act[:] *= 0 keeps the sign of zero
+    case VSS_TEAM_SA: return k < 2 ? action[2 * env + k] : ou;
     case VSS_TEAM_CMA:
-    case VSS_TEAM_DMA: return a.team_action[t][6 * env + k];  // (N,6) and (3N,2): the same 6 floats per field
-    default: return prev;                                      // EXTERNAL: as the caller wrote it
+    case VSS_TEAM_DMA: return action[6 * env + k];
+    case VSS_TEAM_EXTERNAL: return prev;
+    default: return ou;  // OU
   }
 }
 
-// Opponent view: yellow slot k (0..5) after the opponent's call (the restatement of vss_set_view_opponent), given
-// the value the caller left in the buffer and the slot's OU draw.
-VSS_HD float opp_slot(const StepArgs& a, long long env, int k, float prev, float ou) {
-  switch (a.team_mode[1]) {
-    case VSS_TEAM_ZERO: return fmul(ou, 0.0f);  // TeamZero on the drawn buffer: act[:] *= 0 keeps the sign of zero
-    case VSS_TEAM_SA: return k < 2 ? a.team_action[1][2 * env + k] : ou;
-    case VSS_TEAM_CMA:
-    case VSS_TEAM_DMA: return a.team_action[1][6 * env + k];  // (N,6) and (3N,2): the same 6 floats per field
-    case VSS_TEAM_EXTERNAL: return prev;                      // as the caller wrote it before the step
-    default: return ou;                                        // OU
+// The slots 4b .. 4b+3 (robots 2b, 2b+1) that drive the step, un-clamped (vss.py:180-187; wrappers.py:102-103), in
+// place: `act` holds the block's OU draw where draws_ou (else the loaded values), `prev` the values loaded from the
+// buffer. Full contract: the caller's actions. Views: the OU draw with the learner's policy action in its slots and,
+// with an opponent, the opponent's yellow slots. Match: each team's slots.
+template <int VIEW>
+VSS_HD void action_slots(float act[4], const float prev[4], long long env, const StepArgs& a, int b) {
+  if (VIEW == VIEW_MATCH) {
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const int s = 4 * b + q, t = s >= 6 ? 1 : 0;
+      act[q] = team_slot(a.team_mode[t], a.team_action[t], env, s - 6 * t, prev[q], prev[q], act[q]);
+    }
+  } else if (VIEW != VIEW_FULL) {
+    if (view_base(VIEW) == VSS_VIEW_SA) {  // act_view[:] = action
+      if (b == 0) { act[0] = a.policy_action[2 * env]; act[1] = a.policy_action[2 * env + 1]; }
+    } else {  // cma (N,6) and dma (3N,2): the same 6 contiguous floats per field
+      for (int q = 4 * b; q < 6 && q < 4 * b + 4; ++q) act[q - 4 * b] = a.policy_action[6 * env + q];
+    }
+    if (VIEW >= VIEW_OPP) {  // the opponent's call on act[:, 1] (slots 6..11)
+#pragma unroll
+      for (int q = 0; q < 4; ++q)
+        if (4 * b + q >= 6)
+          act[q] = team_slot(a.team_mode[1], a.team_action[1], env, 4 * b + q - 6, act[q], prev[q], act[q]);
+    }
   }
 }
 
@@ -945,7 +980,7 @@ template <int VIEW>
 VSS_HD void lane_phase1a(float* S, long long env, const StepArgs& a, const DevParams& P, const RngKey& key) {
   // state in: 60 coalesced loads in flight per lane
   load_state(S, a.state, a.ld, env);
-  // actions (vss.py:180-187; wrappers.py:102-103)
+  // actions: the whole row is loaded before any OU work
   float act[VSS_ACT_PER_FIELD];
   {
     const float* ap = (VIEW == VIEW_FULL ? a.actions : a.action_buf) + env * VSS_ACT_PER_FIELD;
@@ -955,33 +990,13 @@ VSS_HD void lane_phase1a(float* S, long long env, const StepArgs& a, const DevPa
       act[4 * q] = v.x; act[4 * q + 1] = v.y; act[4 * q + 2] = v.z; act[4 * q + 3] = v.w;
     }
   }
-  if (VIEW == VIEW_MATCH) {
-    float ou[VSS_ACT_PER_FIELD];
+  float prev[VSS_ACT_PER_FIELD];
 #pragma unroll
-    for (int q = 0; q < VSS_ACT_PER_FIELD; ++q) ou[q] = act[q];
-    if (match_needs_ou(a)) ou_lane(ou, P, key, step_index(a));
+  for (int q = 0; q < VSS_ACT_PER_FIELD; ++q) prev[q] = act[q];
+  if (draws_ou<VIEW>(a)) ou_lane(act, P, key, step_index(a));
 #pragma unroll
-    for (int q = 0; q < VSS_ACT_PER_FIELD; ++q) act[q] = match_slot(a, env, q, act[q], ou[q]);
-    // the buffer keeps the un-clamped values; done rows are NOT zeroed (play_matches carries them over)
-    float* ap = a.action_buf + env * VSS_ACT_PER_FIELD;
-#pragma unroll
-    for (int q = 0; q < 3; ++q) st4(ap + 4 * q, F4{act[4 * q], act[4 * q + 1], act[4 * q + 2], act[4 * q + 3]});
-  } else if (VIEW != VIEW_FULL) {
-    float prev[6];  // (opponent views) the yellow slots as the caller left them
-#pragma unroll
-    for (int q = 0; q < 6; ++q) prev[q] = act[6 + q];
-    ou_lane(act, P, key, step_index(a));  // action_buf = random_ou(action_buf)
-    if (view_base(VIEW) == VSS_VIEW_SA) {     // act_view[:] = action
-      act[0] = a.policy_action[2 * env]; act[1] = a.policy_action[2 * env + 1];
-    } else {  // cma (N,6) and dma (3N,2): the same 6 contiguous floats per field
-#pragma unroll
-      for (int q = 0; q < 6; ++q) act[q] = a.policy_action[6 * env + q];
-    }
-    if (VIEW >= VIEW_OPP) {  // the opponent's call on act[:, 1]
-#pragma unroll
-      for (int q = 0; q < 6; ++q) act[6 + q] = opp_slot(a, env, q, prev[q], act[6 + q]);
-    }
-    // the view keeps the un-clamped buffer (wrappers.py:102-103); done rows are zeroed in phase 5
+  for (int b = 0; b < 3; ++b) action_slots<VIEW>(act + 4 * b, prev + 4 * b, env, a, b);
+  if (VIEW != VIEW_FULL) {  // the buffer keeps the un-clamped values (views zero done rows in phase 5, a match does not)
     float* ap = a.action_buf + env * VSS_ACT_PER_FIELD;
 #pragma unroll
     for (int q = 0; q < 3; ++q) st4(ap + 4 * q, F4{act[4 * q], act[4 * q + 1], act[4 * q + 2], act[4 * q + 3]});
@@ -1003,8 +1018,7 @@ VSS_HD void lane_phase1a(float* S, long long env, const StepArgs& a, const DevPa
 }
 
 // ---- the same phase 1a in pieces, for the kernel that spreads one tile over several warps -------
-// (k_step_cta: warp j owns bodies j, j+W, ...; body 0-5 = robot, 6 = ball). Together the pieces do
-// exactly what lane_phase1a does, word for word.
+// (k_step_cta: warp j owns bodies j, j+W, ...; body 0-5 = robot, 6 = ball).
 VSS_HD void load_state_words(float* S, const float* state, long long ld, long long env, int w0, int wstep) {
   const float* src = state + env;
   for (int w = w0; w < VSS_STATE_WORDS; w += wstep) S[w * LDS] = ldg(src + (long long)w * ld);
@@ -1013,34 +1027,17 @@ VSS_HD void store_state_words(const float* S, float* state, long long ld, long l
   float* dst = state + env;
   for (int w = w0; w < VSS_STATE_WORDS; w += wstep) dst[(long long)w * ld] = S[w * LDS];
 }
-// Action slots 4b .. 4b+3 of the field (robots 2b, 2b+1): load, OU noise + policy overwrite (views),
-// write-back of the view's buffer, clamp into the state (vss.py:180-187; wrappers.py:102-103).
+// Action slots 4b .. 4b+3 of the field (robots 2b, 2b+1): load, action_slots, write-back of the buffer, clamp into
+// the state.
 template <int VIEW>
 VSS_HD void actions_block(float* S, long long env, const StepArgs& a, const DevParams& P, const RngKey& key, int b) {
   float* ab = const_cast<float*>(VIEW == VIEW_FULL ? a.actions : a.action_buf) + env * VSS_ACT_PER_FIELD + 4 * b;
   const F4 v = ld4(ab);
   float act[4] = {v.x, v.y, v.z, v.w};
-  if (VIEW == VIEW_MATCH) {
-    float ou[4] = {v.x, v.y, v.z, v.w};
-    if (match_needs_ou(a)) ou_block(ou, P, key, step_index(a), (uint32_t)b);
-#pragma unroll
-    for (int q = 0; q < 4; ++q) act[q] = match_slot(a, env, 4 * b + q, act[q], ou[q]);
-    st4(ab, F4{act[0], act[1], act[2], act[3]});
-  } else if (VIEW != VIEW_FULL) {
-    ou_block(act, P, key, step_index(a), (uint32_t)b);
-    if (view_base(VIEW) == VSS_VIEW_SA) {
-      if (b == 0) { act[0] = a.policy_action[2 * env]; act[1] = a.policy_action[2 * env + 1]; }
-    } else {  // cma (N,6) and dma (3N,2): the same 6 contiguous floats per field
-      for (int q = 4 * b; q < 6 && q < 4 * b + 4; ++q) act[q - 4 * b] = a.policy_action[6 * env + q];
-    }
-    if (VIEW >= VIEW_OPP) {  // the opponent's call on act[:, 1] (slots 6..11)
-      const float prev[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-      for (int q = 0; q < 4; ++q)
-        if (4 * b + q >= 6) act[q] = opp_slot(a, env, 4 * b + q - 6, prev[q], act[q]);
-    }
-    st4(ab, F4{act[0], act[1], act[2], act[3]});
-  }
+  const float prev[4] = {v.x, v.y, v.z, v.w};
+  if (draws_ou<VIEW>(a)) ou_block(act, P, key, step_index(a), (uint32_t)b);
+  action_slots<VIEW>(act, prev, env, a, b);
+  if (VIEW != VIEW_FULL) st4(ab, F4{act[0], act[1], act[2], act[3]});
 #pragma unroll
   for (int k = 0; k < 2; ++k) {
     const int r = 2 * b + k;
@@ -1345,20 +1342,24 @@ VSS_HD void write_obs_fields(const float* T, const uint32_t* tab, int lane, int 
   }
 }
 
+// A policy team's bf16 row of the observation of its robot i in field env (SA / CMA: robot 0 -> row env; DMA: robot
+// i -> row 3 env + i), or -1 for none.
+VSS_HD long long team_row(int mode, long long env, int i) {
+  if (mode == VSS_TEAM_DMA) return 3 * env + i;
+  return i == 0 && (mode == VSS_TEAM_SA || mode == VSS_TEAM_CMA) ? env : -1;
+}
+
 // Match mode: the post-reset observation of the tile's fields (cooperative, all 32 lanes of `parts` warps): the f32
-// (N,2,3,52) obs when a.obs is set, and each policy team's bf16 rows (SA / CMA: robot 0 -> row env; DMA: robot i ->
-// row 3 env + i; the yellow rows are the mirrored obs[:,1] rows). Slots that go nowhere are not gathered.
+// (N,2,3,52) obs when a.obs is set, and each policy team's bf16 rows (the yellow rows are the mirrored obs[:,1]
+// rows). Slots that go nowhere are not gathered.
 VSS_HD void write_match_tile(const float* T, const uint32_t* tab, int lane, int valid, long long env0, const StepArgs& a,
                              int part = 0, int parts = 1) {
   const int total = valid * F4_PER_FIELD;
   for (int f = lane + 32 * part; f < total; f += 32 * parts) {
     const int e = f / F4_PER_FIELD, j = f - e * F4_PER_FIELD;
     const int row = j / F4_PER_ROW, t = row / 3, i = row - 3 * t;
-    const int m = a.team_mode[t];
     void* rows = a.team_rows[t];
-    long long r = -1;  // the team's bf16 row of this slot
-    if (rows && m == VSS_TEAM_DMA) r = 3 * (env0 + e) + i;
-    else if (rows && i == 0 && (m == VSS_TEAM_SA || m == VSS_TEAM_CMA)) r = env0 + e;
+    const long long r = rows ? team_row(a.team_mode[t], env0 + e, i) : -1;  // the team's bf16 row of this slot
     if (!a.obs && r < 0) continue;
     const F4 v = obs_gather(T, tab[j], e);
     if (a.obs) st4(a.obs + 4 * (env0 * F4_PER_FIELD + f), v);
@@ -1368,8 +1369,7 @@ VSS_HD void write_match_tile(const float* T, const uint32_t* tab, int lane, int 
 
 // Opponent view: the yellow team's post-reset observation of the tile's fields (cooperative, all 32 lanes of `parts`
 // warps), gathered through obs-table entries 39..77 (the mirrored obs[:,1] rows): the f32 (N,3,52) rows when
-// a.opp_obs is set, and the policy opponent's bf16 rows (SA / CMA: robot 0 -> row env; DMA: robot i -> row 3 env + i).
-// Only robot 0 is gathered when nothing else goes anywhere.
+// a.opp_obs is set, and the policy opponent's bf16 rows. Only robot 0 is gathered when nothing else goes anywhere.
 VSS_HD void write_opp_tile(const float* T, const uint32_t* tab, int lane, int valid, long long env0, const StepArgs& a,
                            int part = 0, int parts = 1) {
   const int m = a.team_mode[1];
@@ -1382,7 +1382,7 @@ VSS_HD void write_opp_tile(const float* T, const uint32_t* tab, int lane, int va
     const int e = f / per, j = f - e * per, i = j / F4_PER_ROW;
     const F4 v = obs_gather(T, tab[TEAM + j], e);
     if (a.opp_obs) st4(a.opp_obs + 4 * ((env0 + e) * TEAM + j), v);
-    const long long r = m == VSS_TEAM_DMA ? 3 * (env0 + e) + i : (i == 0 ? env0 + e : -1);
+    const long long r = team_row(m, env0 + e, i);
     if (rows && r >= 0) st_bf16x4(rows, r * 64 + (j - i * F4_PER_ROW) * 4, v);
   }
 }

@@ -154,15 +154,7 @@ k_step(const __grid_constant__ StepArgs a, const __grid_constant__ DevParams P) 
   if (SYNC) __syncthreads();
   // 2. terminal observation + observation of the fields that keep their state (vss.py:195-196)
   const uint32_t done_mask = __ballot_sync(0xffffffffu, done);
-  float* ob = a.obs + env0 * (PER_FIELD * 4);
-  float* tob = a.term_obs ? a.term_obs + env0 * (PER_FIELD * 4) : nullptr;
-  // (views only) the same rows as bf16, padded to 64 columns: the tile's first view row is env0 * AGENTS
-  void* obh = (VIEW != VIEW_FULL && a.obs_bf16)
-                  ? static_cast<void*>(static_cast<unsigned short*>(a.obs_bf16) + env0 * (ViewShape<VIEW>::AGENTS * 64))
-                  : nullptr;
-  void* pk = (VIEW != VIEW_FULL && a.packed)
-                 ? static_cast<void*>(static_cast<char*>(a.packed) + env0 * (ViewShape<VIEW>::AGENTS * VSS_PACKED_ROW_BYTES))
-                 : nullptr;
+  const auto [ob, tob, obh, pk] = tile_out<VIEW>(a, env0);
   if (VIEW == VIEW_MATCH) {}  // (no terminal observation: every row is written once, after the reset)
   else if (PER_FIELD >= 32) write_obs_tile_rows<PER_FIELD>(T, tab, lane, valid, tob, ob, done_mask, obh, pk);
   else write_obs_tile(T, tab, lane, valid, PER_FIELD, tob, ob, done_mask, obh, pk);
@@ -323,14 +315,7 @@ k_step_cta(const __grid_constant__ StepArgs a, const __grid_constant__ DevParams
   }
   // 1d. post_physics_step per field (warp 0): progress, rewards, dones, per-field outputs — while the other
   // warps write 2. terminal observation + observation (vss.py:195-196) of all fields
-  float* ob = a.obs + env0 * (PER_FIELD * 4);
-  float* tob = a.term_obs ? a.term_obs + env0 * (PER_FIELD * 4) : nullptr;
-  void* obh = (VIEW != VIEW_FULL && a.obs_bf16)
-                  ? static_cast<void*>(static_cast<unsigned short*>(a.obs_bf16) + env0 * (ViewShape<VIEW>::AGENTS * 64))
-                  : nullptr;
-  void* pk = (VIEW != VIEW_FULL && a.packed)
-                 ? static_cast<void*>(static_cast<char*>(a.packed) + env0 * (ViewShape<VIEW>::AGENTS * VSS_PACKED_ROW_BYTES))
-                 : nullptr;
+  const auto [ob, tob, obh, pk] = tile_out<VIEW>(a, env0);
   if (warp == 0) {
     int code = LANE_RUNNING;
     if (active) code = lane_outputs<VIEW>(S, env, a, P, finite);

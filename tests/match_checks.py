@@ -14,14 +14,11 @@ through orc.step_view by test_match_emu.py), a table of slot overwrites (play.py
 as is.
 """
 import ctypes as C
-import os
-import subprocess
-import tempfile
 
 import numpy as np
 
 import parity_checks as pc
-from backends import ROOT, EmuBackend, GpuBackend
+from backends import EmuBackend, GpuBackend
 from oracle import vss_oracle as orc
 
 ZERO, OU, SA, CMA, DMA, EXTERNAL = 0, 1, 2, 3, 4, 5
@@ -144,21 +141,7 @@ def assert_board_matches_loop(board, loop, what):
 
 # ------------------------------------------------------------------ backends
 class EmuMatchBackend(EmuBackend):
-    """EmuBackend + the match step of tests/emu/vss_emu_match.cpp (compiled on first use into a temporary directory)."""
-
-    _match_lib = None
-
-    @classmethod
-    def match_lib(cls):
-        if cls._match_lib is None:
-            d = tempfile.mkdtemp(prefix="vss_emu_match_")
-            so = os.path.join(d, "libvss_emu_match.so")
-            src = os.path.join(ROOT, "tests", "emu", "vss_emu_match.cpp")
-            cxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
-            subprocess.run([cxx, "-O2", "-std=c++17", "-fPIC", "-ffp-contract=off", "-fopenmp", "-fvisibility=hidden",
-                            "-shared", "-x", "c++", "-o", so, src, "-lm"], check=True, capture_output=True)
-            cls._match_lib = C.CDLL(so)
-        return cls._match_lib
+    """EmuBackend + the match step of the host emulation (emu_step_match)."""
 
     def step_match(self, modes, acts, action_buf, reset_buf, count_envs, n_matches, board, want_obs=True):
         n = self.n
@@ -166,7 +149,7 @@ class EmuMatchBackend(EmuBackend):
         acts = [None if a is None else np.ascontiguousarray(a, np.float32) for a in acts]
         obs = np.zeros((n, 2, 3, 52), np.float32) if want_obs else None
         mode_arr = np.array(modes, np.int32)
-        rc = self.match_lib().emu_step_match(
+        rc = self.lib().emu_step_match(
             C.byref(self.params), _p(self.state), C.c_longlong(n), C.c_longlong(self.ld), C.c_ulonglong(self.goff),
             C.c_ulonglong(self.seed), C.c_uint(self.step_count & 0xFFFFFFFF), _p(mode_arr), _p(acts[0]), _p(acts[1]),
             _p(rows[0]), _p(rows[1]), _p(action_buf), _p(reset_buf), _p(obs), C.c_longlong(count_envs),

@@ -15,15 +15,12 @@ teams (which stores the draw un-clamped and keeps done rows): it is the kernel's
 bit for bit. That draw is itself checked against match_checks.ou_draw (the numpy restatement) within 2e-6 (libm).
 """
 import ctypes as C
-import os
-import subprocess
-import tempfile
 
 import numpy as np
 
 import match_checks as mc
 import parity_checks as pc
-from backends import ROOT, VIEW_CMA, VIEW_DMA, VIEW_SA, EmuBackend, GpuBackend
+from backends import VIEW_CMA, VIEW_DMA, VIEW_SA, EmuBackend, GpuBackend
 from oracle import vss_oracle as orc
 
 ZERO, OU, SA, CMA, DMA, EXTERNAL = mc.ZERO, mc.OU, mc.SA, mc.CMA, mc.DMA, mc.EXTERNAL
@@ -64,22 +61,7 @@ def predicted_slots(view, mode, pa, opp_act, prev, ou):
 
 # ------------------------------------------------------------------ backends
 class EmuOppBackend(mc.EmuMatchBackend):
-    """EmuBackend + the opponent view step of tests/emu/vss_emu_opp.cpp (compiled on first use into a temporary
-    directory)."""
-
-    _opp_lib = None
-
-    @classmethod
-    def opp_lib(cls):
-        if cls._opp_lib is None:
-            d = tempfile.mkdtemp(prefix="vss_emu_opp_")
-            so = os.path.join(d, "libvss_emu_opp.so")
-            src = os.path.join(ROOT, "tests", "emu", "vss_emu_opp.cpp")
-            cxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
-            subprocess.run([cxx, "-O2", "-std=c++17", "-fPIC", "-ffp-contract=off", "-fopenmp", "-fvisibility=hidden",
-                            "-shared", "-x", "c++", "-o", so, src, "-lm"], check=True, capture_output=True)
-            cls._opp_lib = C.CDLL(so)
-        return cls._opp_lib
+    """EmuBackend + the opponent view step of the host emulation (emu_step_view_opp)."""
 
     def step_view_opp(self, view, policy_action, action_buf, reset_buf, ep_ret, ep_len, mode, opp_action,
                       want_obs=True):
@@ -91,7 +73,7 @@ class EmuOppBackend(mc.EmuMatchBackend):
         rows = z((mc.nv_of(mode, n), 64), np.uint16) if mode in POLICY else None
         opp_obs = z((n, 3, 52), np.float32) if want_obs else None
         oa = None if opp_action is None else np.ascontiguousarray(opp_action, np.float32)
-        rc = self.opp_lib().emu_step_view_opp(
+        rc = self.lib().emu_step_view_opp(
             C.byref(self.params), C.c_int(view), _p(self.state), C.c_longlong(n), C.c_longlong(self.ld),
             C.c_ulonglong(self.goff), C.c_ulonglong(self.seed), C.c_uint(self.step_count & 0xFFFFFFFF), _p(reset_buf),
             _p(out["obs"]), _p(out["term_obs"]), _p(out["rews"]), _p(out["timeout"]), _p(out["progress"]),
