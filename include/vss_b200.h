@@ -350,6 +350,17 @@ VSS_API int vss_set_view_opponent(vss_handle h, const vss_view_opponent* opp);
  * (VSS_STATE_WORDS x ld 32-bit words) device->device. */
 VSS_API int vss_get_state(vss_handle h, float* state_out, void* stream);
 VSS_API int vss_set_state(vss_handle h, const float* state_in, void* stream);
+/* The reference's viewer / RecordVideo frames (ppo…:213-221, play.py:134-142, vss.py:16-23,389,412-417), drawn
+ * from the state on the device: renders fields [first_field, first_field + num_fields) of the current state into
+ * `rgb`, (num_fields, height, width, 3) uint8 RGB, row-major. The picture is exact and defined per pixel in
+ * csrc/vss_render.cuh (DESIGN.md §4.7): field, goals, lines, ball, and the six robots with their team colour
+ * behind and their ID colour in front of the centre; 560 x 720 is 400 px/m. A frame shows the state as it is
+ * (after a step, a field that ended an episode is shown already reset). Reads the state only: no counter or handle
+ * state changes; no synchronisation and no allocation, so a CUDA graph can capture it. Arguments are checked
+ * before anything else (rgb null or not 16-byte aligned; height / width not a multiple of 16 in [64, 4096]; then
+ * the handle; then num_fields >= 1 and the range inside [0, num_envs)). */
+VSS_API int vss_render(vss_handle h, int64_t first_field, int32_t num_fields, int32_t height, int32_t width,
+                       uint8_t* rgb, void* stream);
 /* number of view steps executed so far (keys the OU-noise RNG of the views; vss_step draws no noise
  * and does not advance it). The counter is device-resident and advanced by the step kernel itself — by
  * the CTA that completes the step, counted over all the range launches of that step — so CUDA-graph

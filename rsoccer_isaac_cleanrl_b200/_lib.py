@@ -120,6 +120,7 @@ _SYMBOLS = {
     "vss_step_match": (C.c_int, [_VP, C.POINTER(MatchTeam), _VP, _VP, _VP, C.c_int64, C.c_int64, _VP, _VP]),
     "vss_set_view_opponent": (C.c_int, [_VP, C.POINTER(ViewOpponent)]),
     "vss_get_state": (C.c_int, [_VP, _VP, _VP]),
+    "vss_render": (C.c_int, [_VP, C.c_int64, C.c_int32, C.c_int32, C.c_int32, _VP, _VP]),
     "vss_set_state": (C.c_int, [_VP, _VP, _VP]),
     "vss_step_count": (C.c_uint64, [_VP]),
     "vss_set_step_count": (C.c_int, [_VP, C.c_uint64]),

@@ -20,6 +20,7 @@
 #include <string>
 
 #include "vss_lane.cuh"
+#include "vss_render.cuh"
 
 namespace vss {
 
@@ -454,6 +455,32 @@ k_gae(const float* __restrict__ rewards, const float* __restrict__ values, const
     last = gae_step(gae_load(rewards, values, next_values, next_dones, next_timeouts, i), last, gamma, gamma_lambda,
                     advantages, returns, i);
   }
+}
+
+// ---------------------------------------------------------------------------------------- frames (vss_render)
+// One CTA per (frame, band of RENDER_THREADS 16-pixel segments = a band of rows); the field's RENDER_WORDS state
+// words are read once into shared memory. Each thread draws 16 consecutive pixels of a row (csrc/vss_render.cuh)
+// and stores their 48 bytes with three 16-byte stores: a warp writes 1 536 contiguous bytes of a row.
+constexpr int RENDER_THREADS = 128;
+
+__global__ void __launch_bounds__(RENDER_THREADS)
+k_render(const float* __restrict__ state, long long ld, long long first, int height, int width,
+         long long ctas_per_frame, RenderFrame g, uint8_t* __restrict__ rgb) {
+  __shared__ float f[RENDER_WORDS];
+  const long long frame = blockIdx.x / ctas_per_frame;
+  const int band = (int)(blockIdx.x - frame * ctas_per_frame);
+  if (threadIdx.x < RENDER_WORDS) f[threadIdx.x] = state[(long long)render_word(threadIdx.x) * ld + first + frame];
+  __syncthreads();
+  const int segs_per_row = width >> 4;
+  const int seg = band * RENDER_THREADS + (int)threadIdx.x;
+  if (seg >= height * segs_per_row) return;
+  const int i = seg / segs_per_row, j0 = (seg - i * segs_per_row) << 4;
+  uint32_t w[12];
+  render_segment(g, f, i, j0, w);
+  uint4* out = reinterpret_cast<uint4*>(rgb + ((frame * height + i) * (long long)width + j0) * 3);
+  out[0] = make_uint4(w[0], w[1], w[2], w[3]);
+  out[1] = make_uint4(w[4], w[5], w[6], w[7]);
+  out[2] = make_uint4(w[8], w[9], w[10], w[11]);
 }
 
 }  // namespace vss
@@ -927,6 +954,29 @@ VSS_API int vss_get_state(vss_handle h, float* state_out, void* stream) {
   if (int rc = use_device(h)) return rc;
   VSS_CUDA(cudaMemcpyAsync(state_out, h->state, sizeof(float) * VSS_STATE_WORDS * (size_t)h->ld,
                            cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  return VSS_OK;
+}
+
+VSS_API int vss_render(vss_handle h, int64_t first_field, int32_t num_fields, int32_t height, int32_t width,
+                       uint8_t* rgb, void* stream) {
+  if (!rgb) return fail(VSS_E_INVALID, "vss_render: null rgb");
+  if (reinterpret_cast<uintptr_t>(rgb) & 15u) return fail(VSS_E_INVALID, "vss_render: rgb must be 16-byte aligned");
+  if (height % 16 != 0 || height < 64 || height > 4096)
+    return fail(VSS_E_INVALID, "vss_render: height must be a multiple of 16 in [64, 4096]");
+  if (width % 16 != 0 || width < 64 || width > 4096)
+    return fail(VSS_E_INVALID, "vss_render: width must be a multiple of 16 in [64, 4096]");
+  if (!h) return fail(VSS_E_INVALID, "vss_render: null handle");
+  if (num_fields < 1) return fail(VSS_E_INVALID, "vss_render: num_fields must be >= 1");
+  if (first_field < 0 || first_field > h->n - num_fields)
+    return fail(VSS_E_INVALID, "vss_render: fields outside [0, num_envs)");
+  const long long ctas_per_frame = ((long long)height * (width / 16) + RENDER_THREADS - 1) / RENDER_THREADS;
+  if (ctas_per_frame * num_fields > 0x7FFFFFFFLL)
+    return fail(VSS_E_INVALID, "vss_render: too many pixels for one launch (split the fields)");
+  if (int rc = use_device(h)) return rc;
+  const RenderFrame g = render_frame(h->params, height, width);
+  k_render<<<(unsigned)(ctas_per_frame * num_fields), RENDER_THREADS, 0, (cudaStream_t)stream>>>(
+      h->state, h->ld, first_field, height, width, ctas_per_frame, g, rgb);
+  VSS_CUDA(cudaGetLastError());
   return VSS_OK;
 }
 

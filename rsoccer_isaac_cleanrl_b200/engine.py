@@ -70,6 +70,21 @@ class Engine:
         check(self.lib.vss_set_state(self._h, _ptr(state, torch.float32, _lib.STATE_WORDS * self.ld, "state"),
                                      self._stream()))
 
+    def render(self, first_field, num_fields, height=560, width=720, out=None):
+        """RGB frames (num_fields, height, width, 3) uint8 of fields [first_field, first_field + num_fields) of the
+        current state, rendered on the device on the current stream (include/vss_b200.h: vss_render; the picture
+        is DESIGN.md §4.7). A frame shows the state as it is: after a step, a field that ended an episode is
+        shown already reset. Reads the state only; no synchronisation and, with `out`, no allocation, so it can
+        be captured in a CUDA graph."""
+        shape = (int(num_fields), int(height), int(width), 3)
+        if out is None:
+            out = torch.empty(shape, dtype=torch.uint8, device=self.device)
+        elif tuple(out.shape) != shape:
+            raise ValueError(f"out: expected shape {shape}, got {tuple(out.shape)}")
+        check(self.lib.vss_render(self._h, int(first_field), int(num_fields), int(height), int(width),
+                                  _ptr(out, torch.uint8, name="out"), self._stream()))
+        return out
+
     @property
     def step_count(self):
         return int(self.lib.vss_step_count(self._h))

@@ -163,8 +163,17 @@ class VSS:
         self.extras["time_outs"] = self.timeout_buf.to(self.rl_device)
         return self._obs_out(), self.rew_buf.to(self.rl_device), self.reset_buf.to(self.rl_device), self.extras
 
-    def render(self, mode="rgb_array"):
-        raise NotImplementedError("rendering is out of scope of the B200 engine (SURVEY §2 #22)")
+    def render(self, mode="rgb_array", fields=1, height=560, width=720):
+        """Fields [0, fields) as one (H', W', 3) uint8 numpy picture: each field rendered on the device
+        (Engine.render, DESIGN.md §4.7), laid out by video.mosaic. The picture is the current state: after a
+        step, a field that ended an episode is shown already reset. mode="human" needs a display, which this
+        engine does not have."""
+        if mode != "rgb_array":
+            raise NotImplementedError(f"render mode {mode!r}: only 'rgb_array' is supported (there is no display)")
+        from ..video import mosaic
+        with torch.cuda.device(self.device):
+            frames = self.engine.render(0, fields, height, width)
+            return mosaic(frames).cpu().numpy()
 
     def close(self):
         self.engine.close()

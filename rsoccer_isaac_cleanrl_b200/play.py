@@ -113,12 +113,17 @@ def baseline_teams(base_dir="base_nets", device="cuda:0"):
     return teams
 
 
-def play_matches(envs, blue_team, yellow_team, n_matches, video_path=None, count_envs=1065):
+def play_matches(envs, blue_team, yellow_team, n_matches, video_path=None, count_envs=1065, video_fields=1):
     """Mean blue goal score and mean episode length over `n_matches` finished episodes
     (reference play.py:131-164). Only the first `count_envs` fields are counted, as the
-    reference does (hard-coded 1065 there)."""
+    reference does (hard-coded 1065 there). With `video_path`, fields [0, video_fields) are rendered after every
+    step (one mp4 frame per loop iteration, several fields as a mosaic; the state after the step: a field that
+    ended an episode is shown already reset)."""
+    writer = None
     if video_path:
-        raise NotImplementedError("video capture is out of scope of the B200 engine")
+        from .video import HEIGHT, WIDTH, VideoWriter
+        writer = VideoWriter(video_path)
+        frame = torch.empty((int(video_fields), HEIGHT, WIDTH, 3), dtype=torch.uint8, device=envs.device)
     envs.reset_buf[:] = 1
     envs.reset_dones()
     ep_count = 0
@@ -133,11 +138,15 @@ def play_matches(envs, blue_team, yellow_team, n_matches, video_path=None, count
         yellow_team(action_buf[:, 1], obs[:, 1])
         obs, rew, dones, info = envs.step(action_buf)
         obs = obs["obs"]
+        if writer is not None:
+            writer.write_frames(envs.engine.render(0, video_fields, HEIGHT, WIDTH, out=frame)[None])
         env_ids = dones[:count_envs].nonzero(as_tuple=False).squeeze(-1)
         if len(env_ids):
             ep_count += len(env_ids)
             rew_sum += rew[env_ids, 0, 0, 0].sum().item()
             len_sum += info["progress_buffer"][env_ids].sum().item()
+    if writer is not None:
+        writer.close()
     return rew_sum / ep_count, len_sum / ep_count
 
 
@@ -193,10 +202,15 @@ class _DevicePolicy:
                                         call_offset=call_offset, action=self.action, logprob=self.logprob))
 
 
-def _run_matches_fused(envs, blue_team, yellow_team, n_matches, count_envs=1065, seed=0, graphs=True):
-    """play_matches_fused with its scoreboard: dict(score, length, matches, steps, buffers). `buffers` holds the final
-    action buffer and the policy teams' last sampled actions. graphs=False runs every chunk eagerly: the same
-    launches in the same order, which the tests compare the graph replays against."""
+def _run_matches_fused(envs, blue_team, yellow_team, n_matches, count_envs=1065, seed=0, graphs=True, video_path=None,
+                       video_fields=1):
+    """play_matches_fused with its scoreboard: dict(score, length, matches, steps, video_frames, buffers). `buffers`
+    holds the final action buffer, the policy teams' last sampled actions and, with a video, the last chunk's device
+    frames (K, F, H, W, 3). graphs=False runs every chunk eagerly: the same launches in the same order, which the
+    tests compare the graph replays against. With `video_path` every chunk also renders fields [0, video_fields)
+    after each step (inside the captured graph) and the host writes the chunk's frames after it: the video holds
+    every executed step, the steps a chunk runs past the end of the evaluation included; video_frames counts them.
+    Without a video the launches are exactly those of a run without the feature."""
     n = envs.num_fields
     dev = envs.device
     count_envs = min(int(count_envs), n)
@@ -217,6 +231,21 @@ def _run_matches_fused(envs, blue_team, yellow_team, n_matches, count_envs=1065,
         obs = envs.obs_buf if external else None
         specs = [(m, None if p is None else p.action, None if p is None else p.rows) for m, p in zip(modes, pol)]
         side_stream = torch.cuda.Stream(device=dev)
+        writer = frames = None
+        if video_path:
+            from .video import HEIGHT, WIDTH, VideoWriter
+            writer = VideoWriter(video_path)
+            frames = torch.zeros((_CHUNK, int(video_fields), HEIGHT, WIDTH, 3), dtype=torch.uint8, device=dev)
+        shown = [0]  # frames of the last chunk (all _CHUNK except, on the EXTERNAL path, possibly the last)
+
+        def render(k):
+            if frames is not None:
+                envs.engine.render(0, frames.shape[1], frames.shape[2], frames.shape[3], out=frames[k])
+
+        def flush(k):
+            if writer is not None and k:
+                writer.write_frames(frames[:k])
+                shown[0] = k
 
         def policies(call_offset):
             active = [p for p in pol if p is not None]
@@ -240,6 +269,7 @@ def _run_matches_fused(envs, blue_team, yellow_team, n_matches, count_envs=1065,
             return (int(board[4].item()) & 0xFFFFFFFF) != 0
 
         if external:  # EXTERNAL teams run eagerly on the step's f32 observation: no graph, one check per step
+            k = 0
             while not frozen():
                 for side, (t, m) in enumerate(zip(teams, modes)):
                     if m == _lib.TEAM_EXTERNAL:
@@ -248,18 +278,27 @@ def _run_matches_fused(envs, blue_team, yellow_team, n_matches, count_envs=1065,
                 for p in pol:
                     if p is not None:
                         p.counter.add_(1)
+                render(k)
+                k += 1
+                if k == _CHUNK:
+                    flush(k)
+                    k = 0
+            flush(k)
         else:
             def chunk():
                 for k in range(_CHUNK):
                     step(k)
+                    render(k)
                 for p in pol:
                     if p is not None:
                         p.counter.add_(_CHUNK)
 
             chunk()  # eager first chunk (also the warm-up of everything the graph records)
+            flush(_CHUNK)
             if not graphs:
                 while not frozen():
                     chunk()
+                    flush(_CHUNK)
             elif not frozen():
                 torch.cuda.synchronize(dev)
                 graph = torch.cuda.CUDAGraph()
@@ -267,23 +306,32 @@ def _run_matches_fused(envs, blue_team, yellow_team, n_matches, count_envs=1065,
                     chunk()
                 while True:
                     graph.replay()
+                    flush(_CHUNK)
                     if frozen():
                         break
         b = board.cpu()
+        if writer is not None:
+            writer.close()
     envs._obs_stale = True  # the step wrote neither obs_buf (unless EXTERNAL) nor the reward / terminal buffers
     matches = int(b[0])
     return dict(score=float(b[2:3].view(torch.float64)[0]) / matches, length=int(b[1]) / matches, matches=matches,
-                steps=int(b[3]), buffers=dict(action_buf=action_buf, policy_action=[p and p.action for p in pol]))
+                steps=int(b[3]), video_frames=writer.frames if writer is not None else 0,
+                buffers=dict(action_buf=action_buf, policy_action=[p and p.action for p in pol],
+                             frames=None if frames is None else frames[:shown[0]]))
 
 
-def play_matches_fused(envs, blue_team, yellow_team, n_matches, count_envs=1065, seed=0):
+def play_matches_fused(envs, blue_team, yellow_team, n_matches, count_envs=1065, seed=0, video_path=None,
+                       video_fields=1):
     """play_matches on the device: (mean blue goal score, mean episode length) over the first `n_matches`
     episodes that end among the first `count_envs` fields, exactly as play_matches defines them. TeamZero /
     TeamOU / TeamSA / TeamCMA / TeamDMA run inside the step (policy teams: the actor only, from bf16 copies of
     team.agent's weights, sampled in the same launch); any other team callable runs eagerly on the step's f32
     observation. The teams' OU noise comes from the engine's counter-based stream and the policy noise from a
-    per-team Philox stream derived from `seed`, so results match play_matches in distribution, not draw for draw."""
-    r = _run_matches_fused(envs, blue_team, yellow_team, n_matches, count_envs, seed)
+    per-team Philox stream derived from `seed`, so results match play_matches in distribution, not draw for draw.
+    With `video_path`, fields [0, video_fields) are rendered on the device after every executed step (inside the
+    captured chunks; a frame is the state after its step) and written as an mp4 (see _run_matches_fused)."""
+    r = _run_matches_fused(envs, blue_team, yellow_team, n_matches, count_envs, seed, video_path=video_path,
+                           video_fields=video_fields)
     return r["score"], r["length"]
 
 
@@ -303,6 +351,9 @@ def main(argv=None):
     ap.add_argument("--matches", type=int, default=10000)
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--eager", action="store_true", help="run play_matches (the reference loop) instead")
+    ap.add_argument("--video", default=None, metavar="DIR",
+                    help="write one mp4 per opponent, DIR/<blue>_vs_<yellow>.mp4, of every step of fields [0, F)")
+    ap.add_argument("--video-fields", type=int, default=1, metavar="F", help="fields per video frame (a mosaic)")
     args = ap.parse_args(argv)
     from .envs import VSS, load_cfg
     cfg = load_cfg()
@@ -317,6 +368,10 @@ def main(argv=None):
         opponents = {f"{algo}/{s}": t for algo, by_seed in baseline_teams(args.base_dir).items()
                      for s, t in by_seed.items()}
     for name, yellow in opponents.items():
+        video = None
+        if args.video:
+            from .video import safe_name
+            video = os.path.join(args.video, f"{safe_name(args.blue)}_vs_{safe_name(name)}.mp4")
         torch.cuda.synchronize()
         t0 = time.perf_counter()
         if args.eager:
@@ -325,14 +380,18 @@ def main(argv=None):
             def counted(act, obs, team=blue):
                 steps[0] += 1
                 team(act, obs)
-            score, length = play_matches(envs, counted, yellow, args.matches, count_envs=args.num_envs)
+            score, length = play_matches(envs, counted, yellow, args.matches, count_envs=args.num_envs,
+                                         video_path=video, video_fields=args.video_fields)
             r = dict(score=score, length=length, matches=args.matches, steps=steps[0])
         else:
-            f = _run_matches_fused(envs, blue, yellow, args.matches, count_envs=args.num_envs, seed=args.seed)
+            f = _run_matches_fused(envs, blue, yellow, args.matches, count_envs=args.num_envs, seed=args.seed,
+                                   video_path=video, video_fields=args.video_fields)
             r = dict(score=f["score"], length=f["length"], matches=args.matches, steps=f["steps"],
                      counted_matches=f["matches"])  # (the step that reaches the count adds all its episodes)
         torch.cuda.synchronize()
         r["seconds"] = time.perf_counter() - t0
+        if video:
+            r["video"] = video
         print(json.dumps(dict(blue=args.blue, yellow=name, path="eager" if args.eager else "fused", **r)), flush=True)
 
 

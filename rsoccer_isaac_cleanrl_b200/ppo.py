@@ -71,7 +71,9 @@ def parse_args(argv=None):
     p.add_argument("--target-kl", type=float, default=None)
     p.add_argument("--threshold-kl", type=float, default=0.008)
     p.add_argument("--reward-scaler", type=float, default=1000)  # parsed and unused, as in the reference
-    p.add_argument("--record-video-step-frequency", type=int, default=20000)
+    p.add_argument("--record-video-step-frequency", type=int, default=20000,
+                   help="--capture-video: an update records when its rollout holds a vector-step index k (counted from "
+                        "0, one per env step) with k %% this == 0")
     p.add_argument("--test", type=b, default=False, nargs="?", const=True)
     # engine-specific additions
     p.add_argument("--save-path", type=str, default="runs")
@@ -87,6 +89,8 @@ def parse_args(argv=None):
                         "of the learner) or ppo-sa|ppo-sa-x3|ppo-cma|ppo-dma:PATH (a checkpoint)")
     p.add_argument("--opponent-refresh", type=int, default=10,
                    help="--opponent self: the snapshot is taken before update 1 and then every K updates")
+    p.add_argument("--video-fields", type=int, default=1,
+                   help="--capture-video: fields [0, F) of rank 0, one mosaic per step")
     p.add_argument("--quiet", type=b, default=False, nargs="?", const=True)
     p.add_argument("--tensorboard", type=b, default=True, nargs="?", const=True,
                    help="write the reference's scalar tags (losses/*, Charts/SPS, rws/episodic_*) with SummaryWriter")
@@ -289,17 +293,18 @@ def update_policy(args, batch_size, randperm, run_minibatch, optimizer, read_kl)
 
 
 
+def _run_name(args):
+    return f"{args.exp_name}_ppo-{args.env_id}_{args.seed}"
+
+
 def _make_writer(args, rank, log):
     """SummaryWriter of ppo…:195-199 (rank 0; None when --quiet, --tensorboard false or tensorboard is not
-    installed). W&B (--track) and video capture are out of scope (SURVEY §2 #18, #22): say so instead of
-    silently ignoring the flags."""
+    installed). W&B (--track) is out of scope (SURVEY §2 #18): say so instead of silently ignoring the flag."""
     if rank != 0:
         return None
     if args.track:
         log("warning: --track (Weights & Biases) is not implemented by this engine; the TensorBoard event file "
             "carries the same scalars")
-    if args.capture_video:
-        log("warning: --capture-video is not implemented by this engine (no renderer); flag ignored")
     if args.quiet or not getattr(args, "tensorboard", True):
         return None
     try:
@@ -307,8 +312,7 @@ def _make_writer(args, rank, log):
     except Exception as e:
         log(f"warning: tensorboard is not available ({e}); no event file is written")
         return None
-    run_name = f"{args.exp_name}_ppo-{args.env_id}_{args.seed}"
-    writer = SummaryWriter(os.path.join(getattr(args, "save_path", "runs"), run_name))
+    writer = SummaryWriter(os.path.join(getattr(args, "save_path", "runs"), _run_name(args)))
     writer.add_text("hyperparameters", "|param|value|\n|-|-|\n%s" % (
         "\n".join([f"|{key}|{value}|" for key, value in vars(args).items()])))
     return writer
@@ -450,7 +454,13 @@ def train(args, log=print, hook=None):
         term_count = torch.zeros(1, device=device, dtype=torch.int32)
         term_values = torch.zeros(term_cap, device=device, dtype=torch.float32)
 
-    def rollout_fused(first_obs):
+    def render_after_step(frames, step):
+        """--capture-video: the fields of the recorded video after env step `step` (the state after the step: a field
+        that ended an episode is shown already reset)."""
+        if frames is not None:
+            unwrapped_env.engine.render(0, frames.shape[1], frames.shape[2], frames.shape[3], out=frames[step])
+
+    def rollout_fused(first_obs, frames=None):
         """rollout() as two launches per step: the fused MLP forward (both networks' four tcgen05 layers + heads,
         action sample and log-prob written into the rollout slabs, the critic's value into values[step]) and the env
         step (obs / reward / done / timeout slabs and the next bf16 MLP input)."""
@@ -483,6 +493,7 @@ def train(args, log=print, hook=None):
                           reward_out=rewards[step], obs_bf16_out=x16_buf[(step + 1) & 1],
                           done_f_out=next_dones[step], timeout_f_out=next_timeouts[step],
                           opponent_issued=opp_dev is not None)
+                render_after_step(frames, step)
                 if not one_launch:
                     join_side()
             sample_ctr.add_(T)
@@ -503,11 +514,11 @@ def train(args, log=print, hook=None):
                        advantages, returns)
         return obs_all[T]
 
-    def rollout(first_obs):
+    def rollout(first_obs, frames=None):
         """T env steps + V(terminal obs) + GAE (ppo…:256-296). No host sync anywhere, so the whole
-        thing can be captured in a CUDA graph."""
+        thing can be captured in a CUDA graph. With `frames` (T, F, H, W, 3) uint8, one render after each env step."""
         if fused:
-            return rollout_fused(first_obs)
+            return rollout_fused(first_obs, frames)
         with torch.no_grad():
             obs_all[0] = first_obs
             for step in range(T):
@@ -521,6 +532,7 @@ def train(args, log=print, hook=None):
                                                   term_obs_out=term_obs_all[step], reward_out=rewards[step])
                 next_dones[step] = next_done
                 next_timeouts[step] = info["time_outs"]
+                render_after_step(frames, step)
             cur = obs_all[T]
             # V(terminal_observation) for the whole rollout in one batched pass (ppo…:272 does it per step)
             next_values.copy_(agent.get_value(term_obs_all.view(T * N, *oshape)).view(T, N))
@@ -613,6 +625,24 @@ def train(args, log=print, hook=None):
         clip_and_step()
 
     rollout_graph = None
+    # --capture-video (rank 0): a recording update runs the same rollout plus one render after each env step into
+    # `frames`; from update 2 on that is a second captured graph, so the plain rollout graph stays as it is
+    capture = bool(getattr(args, "capture_video", False)) and rank == 0
+    video_freq = max(1, int(getattr(args, "record_video_step_frequency", 20000)))
+    video_dir = os.path.join(getattr(args, "save_path", "runs"), _run_name(args), "videos")
+    if capture:
+        from .video import HEIGHT, WIDTH
+        frames = torch.zeros((T, int(getattr(args, "video_fields", 1)), HEIGHT, WIDTH, 3), dtype=torch.uint8,
+                             device=device)
+    else:
+        frames = None
+    record_graph = None
+
+    def records(update):
+        """Does the rollout of `update` hold a vector-step index k = (update - 1) T .. update T - 1 with k % freq == 0?"""
+        k0 = (update - 1) * T
+        return capture and -(-k0 // video_freq) * video_freq < k0 + T
+
     mb_graph = fb_graph = opt_graph = None
     state = {"update": 0}
 
@@ -672,7 +702,8 @@ def train(args, log=print, hook=None):
     start_time = time.time()
     next_obs = envs.reset()
     num_updates = args.total_timesteps // (args.batch_size * world)
-    stats = {"sps": [], "updates": 0, "update_wall": [], "rollout_wall": [], "lr": [], "minibatches": [], "epochs": []}
+    stats = {"sps": [], "updates": 0, "update_wall": [], "rollout_wall": [], "lr": [], "minibatches": [], "epochs": [],
+             "videos": []}
     t_roll = t_upd = 0.0
     for update in range(1, num_updates + 1):
         state["update"] = update
@@ -684,7 +715,15 @@ def train(args, log=print, hook=None):
             optimizer.param_groups[0]["lr"] = anneal_lr(update, num_updates, args.learning_rate)
         tr0 = time.time()
         global_step += T * N * world
-        if rollout_graph is not None:
+        record = records(update)
+        if record and args.cuda_graph and update >= 2:
+            if record_graph is None:  # the rollout graph's twin, with the renders
+                torch.cuda.synchronize()
+                record_graph = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(record_graph):
+                    rollout(next_obs, frames)
+            record_graph.replay()
+        elif rollout_graph is not None:
             rollout_graph.replay()
         elif args.cuda_graph and update >= 2:
             # every buffer the rollout touches is static by now (next_obs is the view's own output
@@ -695,7 +734,7 @@ def train(args, log=print, hook=None):
                 rollout(next_obs)
             rollout_graph.replay()
         else:
-            next_obs = rollout(next_obs)
+            next_obs = rollout(next_obs, frames if record else None)
         torch.cuda.synchronize()
         tu0 = time.time()
         t_roll += tu0 - tr0
@@ -713,12 +752,19 @@ def train(args, log=print, hook=None):
             hook(update, dict(obs=obs_all, actions=actions, logprobs=logprobs, rewards=rewards, values=values,
                               next_values=next_values, advantages=advantages, returns=returns, flat=flat,
                               flat_grad=flat_grad, term_obs=term_obs_all, next_dones=next_dones,
-                              agent=agent, env=unwrapped_env, stats=mb_stats, opponent=opp))
+                              agent=agent, env=unwrapped_env, stats=mb_stats, opponent=opp,
+                              frames=frames if record else None))
         stats["rollout_wall"].append(tu0 - tr0)
         stats["update_wall"].append(time.time() - tu0)
         sps = int(global_step / (time.time() - start_time))
         stats["sps"].append(sps)
         stats["updates"] = update
+        if record:  # all T steps of the rollout, one video per recording update
+            from .video import VideoWriter
+            path = os.path.join(video_dir, f"update-{update:06d}.mp4")
+            with VideoWriter(path) as vw:
+                vw.write_frames(frames)
+            stats["videos"].append(path)
         if writer is not None:  # the reference's tags (ppo…:273-279, 367-376); one host read per update
             writer.add_scalar("losses/learning_rate", optimizer.param_groups[0]["lr"], global_step)
             writer.add_scalar("losses/value_loss", mb_stats["v_loss"].item(), global_step)
